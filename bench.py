@@ -4,6 +4,11 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (one process per GPU)
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's own CPU implementation (oracle/_ref)
     python bench.py --check                                        # bench-shape loss parity: CUDA arm vs the fp64 oracle
+    python bench.py --steps K --dump-outputs DIR                   # + the last timed step's losses and gradients as .npy
+
+The library is the one build() left in the tree: bench.py compiles nothing, and refuses a library that was not built from
+the sources as they are now.  The inputs, the weights and the sampling seeds of the timed steps depend only on the
+arguments, so two builds run with the same arguments can be compared output for output.
 
 Headline workload (BASELINE.json configs[1], the configuration the metric is quoted on for one GPU): Pix3D head,
 random-init, batch 32 of synthetic 24^3 blob voxel probabilities (threshold 0.2) + 32 x 256 x 12 x 12 RoI feature maps for
@@ -228,14 +233,41 @@ def timed_resident(wl, pool, steps, flush, sync_all):
     ev = pool.take(steps)
     sync_all()
     l0 = _lib.launch_count
-    for a, b in ev:
+    for i, (a, b) in enumerate(ev):
         flush.zero_()                      # L2 flush between timed iterations (outside the event bracket)
         a.record()
-        wl.step()
+        losses = wl.step()
+        if i == steps - 1:
+            last = {k: v.detach() for k, v in losses.items()}
+        # the graph keeps tensors of the step alive: freed inside the bracket, so the next step does not allocate around it
+        del losses
         b.record()
     sync_all()
     launches = (_lib.launch_count - l0) // steps
-    return [a.elapsed_time(b) for a, b in ev], launches
+    return [a.elapsed_time(b) for a, b in ev], launches, last
+
+
+def step_outputs(wl, losses):
+    """What the last step handed its caller, as host float32 arrays: the three losses and, from backward, the gradient of
+    every refinement weight and of the feature maps (this rank's shard)."""
+    out = {k: v.float().cpu().numpy() for k, v in losses.items()}
+    for i, f in enumerate(wl.fmaps_d):
+        out["feature_map%d.grad" % i] = f.grad.float().cpu().numpy()
+    for name, p in wl.head.named_parameters():
+        if p.grad is not None:
+            out[name + ".grad"] = p.grad.float().cpu().numpy()
+    return out
+
+
+def dump_outputs(arrays, path, limit=64 << 20):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        raise SystemExit("bench.py: %d bytes of outputs exceed the %d-byte dump limit" % (total, limit))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    log("[bench] wrote %d arrays (%d bytes) to %s" % (len(arrays), total, path))
 
 
 def timed_e2e(wl, pool, steps, warmup, flush, sync_all):
@@ -418,7 +450,7 @@ def extra_shapenet_shard(dev, rank, world, pool, flush, sync_all, steps, peaks):
     for _ in range(3):
         wl.step()
     sync_all()
-    ms, launches = timed_resident(wl, pool, steps, flush, sync_all)
+    ms, launches, _ = timed_resident(wl, pool, steps, flush, sync_all)
     total = reduce_max_ms(sum(ms), dev, world)
     out = None
     if rank == 0:
@@ -443,7 +475,7 @@ def extra_bf16_maps(dev, rank, world, pool, flush, sync_all, steps):
     for _ in range(3):
         wl.step()
     sync_all()
-    ms, launches = timed_resident(wl, pool, steps, flush, sync_all)
+    ms, launches, _ = timed_resident(wl, pool, steps, flush, sync_all)
     total = reduce_max_ms(sum(ms), dev, world)
     out = None
     if rank == 0:
@@ -556,9 +588,18 @@ def extra_chamfer_sweep(dev, rank, world, pool, flush, sync_all, fma_peak, reps=
 # ---------------------------------------------------------------------------------------------------------------
 # the CUDA arm
 # ---------------------------------------------------------------------------------------------------------------
+def load_built_library():
+    """The library build() left in the tree.  Nothing is compiled here (the tree may be read-only); a library built from other
+    sources than the tree's would be timed and dumped in their place, so it is refused."""
+    from meshrcnn_b200 import _lib, build
+    if build.needs_build():
+        raise SystemExit("bench.py: %s is missing or was not built from the sources in this tree -- run build() "
+                         "(python -m meshrcnn_b200.build) first" % build.LIB)
+    return _lib.load()
+
+
 def run_cuda(args):
     import torch.distributed as dist
-    from meshrcnn_b200 import _lib, build
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -570,11 +611,7 @@ def run_cuda(args):
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
-    if rank == 0:
-        build.build()
-    if world > 1:
-        dist.barrier()
-    _lib.load()
+    load_built_library()
     steps, warmup = args.steps, max(args.warmup, 3)
 
     def sync_all():
@@ -631,7 +668,12 @@ def run_cuda(args):
     sync_all()
 
     # ---- timed region 1: inputs resident in HBM ----------------------------------------------------------------
-    res_ms, launches = timed_resident(wl, pool, steps, flush, sync_all)
+    # Every step draws its surface-sampling seeds from torch's generator and the start-up loop runs a wall-clock-dependent
+    # number of steps: reseeding here gives the timed steps the same draws on every run (--dump-outputs compares builds).
+    torch.manual_seed(0)
+    res_ms, launches, last_losses = timed_resident(wl, pool, steps, flush, sync_all)
+    outputs = step_outputs(wl, last_losses) if args.dump_outputs and rank == 0 else None
+    del last_losses
     log("[bench] per-step ms (resident):", " ".join("%.2f" % x for x in res_ms))
     # ---- timed region 2: end to end through the module API from pinned host memory --------------------------------
     e2e_ms, phases, host_losses = timed_e2e(wl, pool, steps, max(warmup, E2E_WARMUP_MIN), flush, sync_all)
@@ -722,6 +764,8 @@ def run_cuda(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     if result is not None:
         emit(result)
 
@@ -928,10 +972,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="cpu_baseline", action="store_false")
     ap.add_argument("--no-extras", dest="extras", action="store_false", help="skip BASELINE configs[2..4]")
     ap.add_argument("--check", action="store_true", help="bench-shape loss parity against the fp64 oracle, then exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the losses and gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.check or args.impl != "b200"):
+        ap.error("--dump-outputs dumps the timed steps of the CUDA arm; it does not go with --check or --impl reference")
     if args.check:
-        from meshrcnn_b200 import build
-        build.build()
+        load_built_library()
         emit({"check": "bench-shape losses vs fp64 oracle", "ok": True, **check_bench_shape_losses()})
     elif args.impl == "reference":
         run_reference(args)

@@ -2,9 +2,10 @@
 library is a plain C-ABI shared object (``include/meshrcnn_b200.h``); cudart is linked statically so the
 nvcc-12.9 objects do not depend on the cu128 runtime bundled with torch.
 
-    python -m meshrcnn_b200.build            # (re)build if any source is newer than the .so
+    python -m meshrcnn_b200.build            # (re)build if the sources differ from those the .so was built from
 """
 import glob
+import hashlib
 import os
 import platform
 import shutil
@@ -18,6 +19,7 @@ CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 LIB = os.path.join(HERE, "libmeshrcnn_b200.so")
 OBJ = os.path.join(HERE, "build")
+STAMP = os.path.join(OBJ, "sources.sha256")         # digest of the inputs the library in the tree was built from
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",
@@ -35,12 +37,25 @@ def sources():
     return sorted(glob.glob(os.path.join(CSRC, "*.cu")))
 
 
-def needs_build() -> bool:
-    if not os.path.exists(LIB):
-        return True
-    t = os.path.getmtime(LIB)
+def source_digest() -> str:
+    """SHA-256 over the names and contents of every input of the library and the call shim (and of this file, which holds
+    the flags).  Contents, not timestamps: a tree that was copied, or is read-only, is still judged right."""
+    h = hashlib.sha256()
     deps = sources() + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(os.path.join(ROOT, "include", "*.h"))
-    return any(os.path.getmtime(p) > t for p in deps)
+    for p in sorted(deps + [FASTCALL_SRC, os.path.abspath(__file__)]):
+        h.update(os.path.relpath(p, ROOT).encode() + b"\0")
+        with open(p, "rb") as f:
+            h.update(f.read())
+    return h.hexdigest()
+
+
+def needs_build() -> bool:
+    """True unless the library in the tree was built from the sources as they are now."""
+    try:
+        with open(STAMP) as f:
+            return not os.path.exists(LIB) or f.read().strip() != source_digest()
+    except OSError:
+        return True
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -71,7 +86,9 @@ def build(force: bool = False, verbose: bool = False) -> str:
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("link failed:\n%s\n%s" % (r.stdout, r.stderr))
-    build_fastcall(force)
+    build_fastcall(force=True)
+    with open(STAMP, "w") as f:
+        f.write(source_digest() + "\n")
     return LIB
 
 

@@ -259,3 +259,53 @@ def test_bench_reference_arm_line_keeps_the_contract():
     assert "BASELINE configs[1]" in d["config"]["workload"] and "1 mesh" in d["cpu_baseline"]["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": "meshes/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "model" not in d["config"]
+
+
+@pytest.mark.parametrize("argv, message", [
+    (["--steps", "0"], "--steps must be at least 1"),
+    (["--impl", "reference", "--dump-outputs", "d"], "does not go with --check or --impl reference"),
+    (["--check", "--dump-outputs", "d"], "does not go with --check or --impl reference")])
+def test_bench_rejects_bad_arguments(argv, message):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and message in r.stderr and r.stdout.strip() == ""
+
+
+def test_bench_refuses_a_library_not_built_from_the_tree(lib, monkeypatch):
+    """bench.py compiles nothing; a library whose recorded source digest differs from the tree's sources (an edited .cu
+    file) is refused instead of being timed and dumped as if it were the current code."""
+    import bench
+    from meshrcnn_b200 import build
+    assert not build.needs_build() and bench.load_built_library() is lib
+    monkeypatch.setattr(build, "source_digest", lambda: "0" * 64)
+    assert build.needs_build()
+    with pytest.raises(SystemExit, match="run build"):
+        bench.load_built_library()
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the last timed step's losses and gradients as float32 .npy files.  The timed steps
+    start from a fixed seed, so the same step recomputed here from the same workload gives the same arrays (up to the order
+    of floating-point sums), while the step before it, which draws other surface samples, does not."""
+    import json
+    import bench
+    d = tmp_path / "out"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                        "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-3000:]
+    assert json.loads(r.stdout)["steps"] == 2
+    got = {p.name[:-4]: np.load(p) for p in d.iterdir()}
+    assert sum(x.nbytes for x in got.values()) <= 64 << 20
+
+    wl = bench.HeadWorkload("pix3d", torch.device("cuda", 0), 0, 1)
+    torch.manual_seed(0)
+    first = {k: float(v) for k, v in wl.step().items()}
+    losses = wl.step()
+    want = {k: v.detach().cpu().numpy() for k, v in losses.items()}
+    want["feature_map0.grad"] = wl.fmaps_d[0].grad.cpu().numpy()
+    want.update({n + ".grad": p.grad.cpu().numpy() for n, p in wl.head.named_parameters()})
+    assert len(want) == 3 + 1 + 21 and set(got) == set(want)
+    for k, w in want.items():
+        assert got[k].dtype == np.float32 and got[k].shape == w.shape and np.isfinite(got[k]).all(), k
+        np.testing.assert_allclose(got[k], w, rtol=1e-4, atol=1e-5 * float(np.abs(w).max()), err_msg=k)
+    assert abs(first["chamfer_loss"] - float(got["chamfer_loss"])) > 1e-4 * abs(first["chamfer_loss"])
