@@ -241,6 +241,28 @@ int mrb_sample_points_bwd(const float* gcloud, const float* cloud, const double*
 int mrb_sample_points_bwd_ld(const float* gcloud, const float* cloud, const double* stats, const int32_t* fidx,
                              const float* w, const long long* faces, const int32_t* v_off, int B, int n, float* gverts,
                              int ld_gverts, double* scratch /* 4 * B doubles */, void* stream);
+/* Eval-side sampling (no backward): the points of mrb_sample_points_fwd for the same randomness (same face choice, weights
+ * and Philox counter), multiplied by scale[b] (scale may be NULL: unscaled, bitwise the `raw` output) and NOT normalised;
+ * normals = unit normal (B-A)x(C-A)/|.| of each point's face (zero vector for a degenerate face); fidx_out = global face id.
+ * points, normals: B x n x 3. */
+int mrb_sample_surface_fwd(const float* verts, const long long* faces, const int32_t* v_off, const int32_t* f_off,
+                           const double* cdf, int B, int n, const float* u, const long long* face_idx, const float* xi2,
+                           const float* xi1, unsigned long long seed, const float* scale, float* points, float* normals,
+                           int32_t* fidx_out, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
+ * Mesh evaluation metrics (the Mesh R-CNN paper's protocol; reported by eval_utils.compare_meshes).
+ *   mrb_mesh_gt_scale  scale[b] = target / longest side of the bounding box of vertices [v_off[b], v_off[b+1]) (exact fp32
+ *                      min / max; zero extent gives inf)
+ *   mrb_mesh_metrics   from the k = 0 outputs of mrb_knn_fwd (d_p, i_p: B x P; d_q, i_q: B x Q) and the unit normals
+ *                      n_p (B x P x 3), n_q (B x Q x 3): out[b][3 + 3T] = Chamfer-L2 (mean d_p + mean d_q), NC, AbsNC
+ *                      (0.5 * (mean n.m + mean m.n) over the nearest neighbours, without / with |.|), then for each of the
+ *                      T <= 8 thresholds tau_host[t] (a HOST array, read during the call): Precision, Recall (100 x share of
+ *                      points with fp32 sqrt(d) < tau) and F1 = 2PR / (P + R + 1e-8).  fp64 sums in a fixed order.
+ */
+int mrb_mesh_gt_scale(const float* verts, const int32_t* v_off, int B, float target, float* scale, void* stream);
+int mrb_mesh_metrics(const float* d_p, const int32_t* i_p, const float* d_q, const int32_t* i_q, const float* n_p,
+                     const float* n_q, int B, int P, int Q, const float* tau_host, int T, float* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Chamfer / k-NN -- replaces batched_point2point_distance (cross branch), batched_chamfer_distance and the topk of

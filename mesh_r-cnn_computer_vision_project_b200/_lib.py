@@ -137,6 +137,7 @@ LAUNCHES = {
     "mrb_gc_gather_fwd": 1, "mrb_gc_gather_bwd": 1, "mrb_head_fwd": 1, "mrb_head_bwd": 1, "mrb_voxel_bce_fwd": 2, "mrb_voxel_bce_bwd": 1, "mrb_normal_loss_total_fwd": 2,
     "mrb_normal_loss_total_bwd": 1, "mrb_scalar_combine": 1, "mrb_scalar_scatter": 1, "mrb_face_areas": 1,
     "mrb_face_area_cdf": 2, "mrb_sample_points_fwd": 2, "mrb_normalize_cloud_fwd": 1, "mrb_sample_points_bwd": 2, "mrb_sample_points_bwd_ld": 2,
+    "mrb_sample_surface_fwd": 1, "mrb_mesh_gt_scale": 1, "mrb_mesh_metrics": 1,
     "mrb_knn_fwd": 3, "mrb_knn_fwd_algo": 4, "mrb_sum_scaled": 2, "mrb_chamfer_bwd": 1, "mrb_normals_fwd": 1, "mrb_normals_fwd_eig": 1, "mrb_normals_bwd": 1, "mrb_normals_bwd_ld": 1,
     "mrb_normal_loss_fwd": 2, "mrb_normal_loss_bwd": 1, "mrb_edge_loss_fwd": 2, "mrb_edge_loss_bwd": 1,
 }

@@ -81,6 +81,53 @@ __device__ __forceinline__ uint4 philox4x32(uint32_t c0, uint32_t c1, uint32_t c
 }
 __device__ __forceinline__ float u01(uint32_t x) { return (float)(x >> 8) * (1.0f / 16777216.0f); }   // [0,1)
 
+// One area-weighted surface draw: global face id, global corner vertex ids and barycentric weights of point i of mesh b
+// (pi = b * n + i), from the injected draws or from Philox(i, b, seed).  Shared by k_sample and k_sample_surface, so both
+// draw the same point for the same randomness.
+struct SurfaceDraw {
+    int f;
+    long long a, b, c;
+    float w0, w1, w2;
+};
+
+__device__ __forceinline__ SurfaceDraw draw_surface_point(const long long* __restrict__ faces, const int32_t* __restrict__ v_off,
+                                                          const int32_t* __restrict__ f_off, const double* __restrict__ cdf,
+                                                          const float* __restrict__ u_in, const long long* __restrict__ fidx_in,
+                                                          const float* __restrict__ xi2_in, const float* __restrict__ xi1_in,
+                                                          unsigned long long seed, int b, int i, size_t pi) {
+    const int fb = f_off[b], fe = f_off[b + 1];
+    float u, xi2, xi1;
+    if (xi2_in) {
+        xi2 = xi2_in[pi]; xi1 = xi1_in[pi]; u = u_in ? u_in[pi] : 0.f;
+    } else {
+        const uint4 r = philox4x32((uint32_t)i, (uint32_t)b, 0x5eedu, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
+        u = u01(r.x); xi2 = u01(r.y); xi1 = u01(r.z);
+    }
+    SurfaceDraw s;
+    if (fidx_in) {
+        s.f = fb + (int)fidx_in[pi];
+    } else {
+        // inverse CDF: first face whose inclusive cumulative area exceeds u * total (multinomial, :16)
+        const double target = (double)u * cdf[fe - 1];
+        int lo = fb, hi = fe - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (cdf[mid] > target) hi = mid; else lo = mid + 1;
+        }
+        s.f = lo;
+    }
+    const long long o = v_off[b];
+    s.a = faces[3 * (size_t)s.f] + o; s.b = faces[3 * (size_t)s.f + 1] + o; s.c = faces[3 * (size_t)s.f + 2] + o;
+    const float r = sqrtf(xi1);                          // :21
+    s.w0 = 1.0f - r; s.w1 = (1.0f - xi2) * r; s.w2 = xi2 * r;   // :23-25
+    return s;
+}
+
+// coordinate d of the drawn point (the weighted sum of mesh_sampling.py:27-35)
+__device__ __forceinline__ float surface_coord(const SurfaceDraw& s, const float* __restrict__ verts, int d) {
+    return fmaf(s.w2, verts[3 * s.c + d], fmaf(s.w1, verts[3 * s.b + d], s.w0 * verts[3 * s.a + d]));
+}
+
 // one thread per sampled point
 __global__ void __launch_bounds__(256) k_sample(const float* __restrict__ verts, const long long* __restrict__ faces,
                                                 const int32_t* __restrict__ v_off, const int32_t* __restrict__ f_off,
@@ -93,36 +140,40 @@ __global__ void __launch_bounds__(256) k_sample(const float* __restrict__ verts,
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const size_t pi = (size_t)b * n + i;
-    const int fb = f_off[b], fe = f_off[b + 1];
-    float u, xi2, xi1;
-    if (xi2_in) {
-        xi2 = xi2_in[pi]; xi1 = xi1_in[pi]; u = u_in ? u_in[pi] : 0.f;
-    } else {
-        const uint4 r = philox4x32((uint32_t)i, (uint32_t)b, 0x5eedu, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
-        u = u01(r.x); xi2 = u01(r.y); xi1 = u01(r.z);
-    }
-    int f;
-    if (fidx_in) {
-        f = fb + (int)fidx_in[pi];
-    } else {
-        // inverse CDF: first face whose inclusive cumulative area exceeds u * total (multinomial, :16)
-        const double target = (double)u * cdf[fe - 1];
-        int lo = fb, hi = fe - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (cdf[mid] > target) hi = mid; else lo = mid + 1;
-        }
-        f = lo;
-    }
-    const long long o = v_off[b];
-    const long long a = faces[3 * (size_t)f] + o, bb = faces[3 * (size_t)f + 1] + o, c = faces[3 * (size_t)f + 2] + o;
-    const float r = sqrtf(xi1);                          // :21
-    const float w0 = 1.0f - r, w1 = (1.0f - xi2) * r, w2 = xi2 * r;   // :23-25
+    const SurfaceDraw s = draw_surface_point(faces, v_off, f_off, cdf, u_in, fidx_in, xi2_in, xi1_in, seed, b, i, pi);
 #pragma unroll
-    for (int d = 0; d < 3; ++d)
-        raw[3 * pi + d] = fmaf(w2, verts[3 * c + d], fmaf(w1, verts[3 * bb + d], w0 * verts[3 * a + d]));
-    fidx_out[pi] = f;
-    w_out[3 * pi] = w0; w_out[3 * pi + 1] = w1; w_out[3 * pi + 2] = w2;
+    for (int d = 0; d < 3; ++d) raw[3 * pi + d] = surface_coord(s, verts, d);
+    fidx_out[pi] = s.f;
+    w_out[3 * pi] = s.w0; w_out[3 * pi + 1] = s.w1; w_out[3 * pi + 2] = s.w2;
+}
+
+// Eval-side sampling (no backward): the k_sample point times an optional per-mesh scale (no unit-ball normalisation), the
+// unit normal (B-A)x(C-A)/|.| of its face (zero vector for a degenerate face) and the global face id.
+__global__ void __launch_bounds__(256) k_sample_surface(const float* __restrict__ verts, const long long* __restrict__ faces,
+                                                        const int32_t* __restrict__ v_off, const int32_t* __restrict__ f_off,
+                                                        const double* __restrict__ cdf, int n,
+                                                        const float* __restrict__ u_in, const long long* __restrict__ fidx_in,
+                                                        const float* __restrict__ xi2_in, const float* __restrict__ xi1_in,
+                                                        unsigned long long seed, const float* __restrict__ scale,
+                                                        float* __restrict__ points, float* __restrict__ normals,
+                                                        int32_t* __restrict__ fidx_out) {
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const size_t pi = (size_t)b * n + i;
+    const SurfaceDraw s = draw_surface_point(faces, v_off, f_off, cdf, u_in, fidx_in, xi2_in, xi1_in, seed, b, i, pi);
+    const float sc = scale ? scale[b] : 1.0f;            // x * 1.0f == x: unscaled points equal k_sample's raw points
+#pragma unroll
+    for (int d = 0; d < 3; ++d) points[3 * pi + d] = sc * surface_coord(s, verts, d);
+    const float ax = verts[3 * s.a], ay = verts[3 * s.a + 1], az = verts[3 * s.a + 2];
+    const float ux = verts[3 * s.b] - ax, uy = verts[3 * s.b + 1] - ay, uz = verts[3 * s.b + 2] - az;
+    const float vx = verts[3 * s.c] - ax, vy = verts[3 * s.c + 1] - ay, vz = verts[3 * s.c + 2] - az;
+    const float nx = uy * vz - uz * vy, ny = uz * vx - ux * vz, nz = ux * vy - uy * vx;
+    const float len = sqrtf(nx * nx + ny * ny + nz * nz);
+    normals[3 * pi] = len > 0.f ? nx / len : 0.f;
+    normals[3 * pi + 1] = len > 0.f ? ny / len : 0.f;
+    normals[3 * pi + 2] = len > 0.f ? nz / len : 0.f;
+    fidx_out[pi] = s.f;
 }
 
 struct Stats {   // per cloud, 8 doubles
@@ -400,6 +451,22 @@ extern "C" int mrb_sample_points_fwd(const float* verts, const long long* faces,
                                                          raw, fidx_out, w_out);
     launch_normalize(raw, B, n, cloud, stats, s);
     return check_launch("sample_points_fwd");
+}
+
+extern "C" int mrb_sample_surface_fwd(const float* verts, const long long* faces, const int32_t* v_off,
+                                      const int32_t* f_off, const double* cdf, int B, int n, const float* u,
+                                      const long long* face_idx, const float* xi2, const float* xi1, unsigned long long seed,
+                                      const float* scale, float* points, float* normals, int32_t* fidx_out, void* stream_) {
+    MRB_REQUIRE(verts && faces && v_off && f_off && points && normals && fidx_out, "sample_surface_fwd: null pointer");
+    MRB_REQUIRE(cdf || face_idx, "sample_surface_fwd: need a CDF or injected face indices");
+    MRB_REQUIRE((xi2 == nullptr) == (xi1 == nullptr), "sample_surface_fwd: xi1/xi2 must be given together");
+    MRB_REQUIRE(face_idx || xi2 == nullptr || u, "sample_surface_fwd: injected xi needs injected u or face_idx");
+    MRB_REQUIRE(B <= 65535, "sample_surface_fwd: batch too large");
+    if (B == 0 || n == 0) return MRB_OK;
+    k_sample_surface<<<dim3(ceil_div(n, 256), B), 256, 0, (cudaStream_t)stream_>>>(verts, faces, v_off, f_off, cdf, n, u, face_idx,
+                                                                                   xi2, xi1, seed, scale, points, normals,
+                                                                                   fidx_out);
+    return check_launch("sample_surface_fwd");
 }
 
 extern "C" int mrb_normalize_cloud_fwd(const float* raw, int B, int n, float* cloud, double* stats, void* stream_) {

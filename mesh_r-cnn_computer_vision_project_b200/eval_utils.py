@@ -10,7 +10,7 @@ Reference semantics kept: ``f_score`` works on a confusion matrix c[i, j] = #(pr
 percentages with the 1e-8 guards of :20-26; ``mesh_precision_recall`` zeroes ALL true positives through the scalar-mask
 assignment ``tp[f1 <= 0.5] = 0`` when the running F0.3 is <= 0.5 (:53-60) and integrates precision over recall with
 the trapezoid rule (sklearn ``auc``: the recall values must be monotonic)."""
-from typing import List, Sequence, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import torch
 from torch import Tensor
@@ -115,11 +115,130 @@ def get_only_max(max_indexes: Sequence[int], voxels: Tensor, vertex_positions: L
 
 
 # ---------------------------------------------------------------------------------------------------------------
+# mesh metrics of the Mesh R-CNN paper (Chamfer-L2, normal consistency, F1@tau on GT-10 scaled surface samples)
+# ---------------------------------------------------------------------------------------------------------------
+def mesh_metric_names(thresholds: Sequence[float]) -> List[str]:
+    """Keys of ``compare_meshes`` in the column order of its per-mesh table."""
+    names = ["Chamfer-L2", "NormalConsistency", "AbsNormalConsistency"]
+    for tau in thresholds:
+        names += ["Precision@%g" % tau, "Recall@%g" % tau, "F1@%g" % tau]
+    return names
+
+
+MESH_METRIC_THRESHOLDS = (0.1, 0.2, 0.3, 0.4, 0.5)
+_PAPER_KEYS = frozenset(mesh_metric_names(MESH_METRIC_THRESHOLDS))
+
+
+def mesh_metric_sums(per_mesh: dict) -> Tuple[List[str], Tensor]:
+    """(metric keys, fp64 [len(keys) + 1]): the sums of every per-mesh metric over the valid meshes, then their count."""
+    valid = per_mesh["valid"]
+    keys = [k for k in per_mesh if k != "valid"]
+    vals = torch.stack([per_mesh[k].double() for k in keys])
+    sums = torch.where(valid.unsqueeze(0), vals, torch.zeros_like(vals)).sum(1)
+    return keys, torch.cat([sums, valid.double().sum().reshape(1)])
+
+
+@torch.no_grad()
+def compare_meshes(pred_verts: Tensor, pred_faces: Tensor, pred_v_index: Sequence[int], pred_f_index: Sequence[int],
+                   gt_verts: Tensor, gt_faces: Tensor, gt_v_index: Sequence[int], gt_f_index: Sequence[int],
+                   num_samples: int = 10000, scale: Optional[str] = "gt-10",
+                   thresholds: Sequence[float] = MESH_METRIC_THRESHOLDS, seed: Optional[int] = None, randomness=None,
+                   reduce: bool = True) -> dict:
+    """The mesh metrics of the Mesh R-CNN paper for packed predicted / ground-truth batches (faces hold per-mesh local ids).
+
+    Both meshes of pair b are sampled at ``num_samples`` area-weighted surface points with the normal of the face each
+    point lies on; with ``scale="gt-10"`` both samples are multiplied by ``10 / longest side of the GT bounding box``
+    (``scale=None``: no scaling).  With d_p / d_q the squared distances to the nearest sample of the other mesh:
+
+    - ``Chamfer-L2`` = mean d_p + mean d_q;
+    - ``NormalConsistency`` = 0.5 (mean n_i . m_nn(i) + mean m_j . n_nn(j)), ``AbsNormalConsistency`` the same with |.|;
+    - ``Precision@tau`` / ``Recall@tau`` = 100 x share of predicted / GT samples with sqrt(d) < tau, ``F1@tau`` =
+      2PR / (P + R + 1e-8) for every threshold (at most 8).
+
+    Cubify emits the two triangles of a quad with opposite winding, so the signed ``NormalConsistency`` of cubified meshes
+    is dominated by that flip; ``AbsNormalConsistency`` is the meaningful one for them.
+
+    B is ``len(gt_f_index)``; shorter prediction lists (Cubify drops trailing empty meshes) are padded with empty meshes.  A
+    predicted mesh without faces is invalid: NaN Chamfer / NC / AbsNC, 0 for P / R / F1.  Randomness: ``seed`` (predicted
+    samples; the GT samples use ``seed + 1``; default: drawn from torch's generator) or ``randomness = (rnd_pred, rnd_gt)``
+    with ``rnd_* = dict(u=|face_idx=, xi2=, xi1=)`` (B x num_samples tensors, rows of invalid meshes ignored).
+
+    Returns ``{key: fp32 tensor [B]}`` plus ``valid`` (bool [B]) with ``reduce=False``; with ``reduce=True`` the 0-dim means
+    over the valid meshes plus ``num_valid`` (int).  No device -> host read."""
+    from . import functional as F_
+    F_._require_cuda(pred_verts, "compare_meshes")
+    F_._require_cuda(gt_verts, "compare_meshes")
+    thresholds = [float(t) for t in thresholds]
+    if len(thresholds) > F_.MAX_THRESHOLDS:
+        raise ValueError("compare_meshes: at most %d thresholds, got %d" % (F_.MAX_THRESHOLDS, len(thresholds)))
+    if scale not in (None, "gt-10"):
+        raise ValueError("compare_meshes: scale must be 'gt-10' or None, got %r" % (scale,))
+    B = len(gt_f_index)
+    if len(gt_v_index) != B:
+        raise ValueError("compare_meshes: gt_v_index and gt_f_index differ in length")
+    if B == 0 or min(gt_f_index) <= 0:
+        raise ValueError("compare_meshes: every ground-truth mesh needs at least one face")
+    if len(pred_v_index) > B or len(pred_f_index) > B:
+        raise ValueError("compare_meshes: %d / %d predicted meshes for %d ground-truth meshes"
+                         % (len(pred_v_index), len(pred_f_index), B))
+    pv = list(pred_v_index) + [0] * (B - len(pred_v_index))
+    pf = list(pred_f_index) + [0] * (B - len(pred_f_index))
+    if sum(pv) != pred_verts.shape[0] or sum(pf) != pred_faces.shape[0]:
+        raise ValueError("compare_meshes: predicted index lists do not match the packed tensors")
+    n = int(num_samples)
+    rnd_pred, rnd_gt = randomness if randomness is not None else ({}, {})
+    if seed is None:
+        seed = 0 if ("xi2" in rnd_pred and "xi2" in rnd_gt) else F_._next_seed()
+
+    valid = [b for b in range(B) if pf[b] > 0]
+    cols = mesh_metric_names(thresholds)
+    dev = pred_verts.device
+    met = rows = None
+    if valid:
+        starts = [0]
+        for c in pv:
+            starts.append(starts[-1] + c)
+        gv, gf, gvi, gfi = gt_verts, gt_faces, list(gt_v_index), list(gt_f_index)
+        if len(valid) < B:
+            # empty predicted meshes occupy no rows: only their offsets drop out; the GT meshes of the pairs are gathered
+            gv = torch.cat([v for b, v in enumerate(gt_verts.split(gvi)) if pf[b] > 0])
+            gf = torch.cat([f for b, f in enumerate(gt_faces.split(gfi)) if pf[b] > 0])
+            gvi, gfi = [gvi[b] for b in valid], [gfi[b] for b in valid]
+            rows = torch.tensor(valid, dtype=torch.int64).to(dev)
+            pick = lambda r: {k: (t.to(dev)[rows] if isinstance(t, Tensor) else t) for k, t in r.items()}
+            rnd_pred, rnd_gt = pick(rnd_pred), pick(rnd_gt)
+        s = F_.mesh_gt_scale(gv, gvi, 10.0) if scale == "gt-10" else None
+        p, n_p, _ = F_.sample_surface(pred_verts, pred_faces, [pv[b] for b in valid], [pf[b] for b in valid], n,
+                                      seed=int(seed), scale=s, v_starts=[starts[b] for b in valid], **rnd_pred)
+        q, n_q, _ = F_.sample_surface(gv, gf, gvi, gfi, n, seed=int(seed) + 1, scale=s, **rnd_gt)
+        d_p, i_p, _, d_q, i_q, _ = F_.knn_search(p, q, 0)
+        met = F_.mesh_metrics(d_p, i_p, d_q, i_q, n_p, n_q, thresholds)
+    if len(valid) == B:
+        table = met
+    else:
+        table = torch.empty(B, len(cols), dtype=torch.float32, device=dev)
+        table[:, :3] = float("nan")
+        table[:, 3:] = 0.0
+        if met is not None:
+            table[rows] = met
+    per_mesh = {k: table[:, i] for i, k in enumerate(cols)}
+    per_mesh["valid"] = torch.tensor([pf[b] > 0 for b in range(B)]).to(dev)
+    if not reduce:
+        return per_mesh
+    keys, sums = mesh_metric_sums(per_mesh)
+    means = (sums[:-1] / len(valid)).float() if valid else torch.full((len(keys),), float("nan"), device=dev)
+    out = {k: means[i] for i, k in enumerate(keys)}
+    out["num_valid"] = len(valid)
+    return out
+
+
+# ---------------------------------------------------------------------------------------------------------------
 # validate on the device path (reference utils/eval_utils.py:93-194)
 # ---------------------------------------------------------------------------------------------------------------
 @torch.no_grad()
 def validate_batch(model_output: dict, batch, point_cloud_size: float = 10e3, num_neighbours_for_normal_loss: int = 10,
-                   f1_thresholds: Sequence[float] = (0.1, 0.3, 0.5), randomness=None, f1_seed: int = 0) -> dict:
+                   f1_thresholds: Sequence[float] = (0.1, 0.3, 0.5), randomness=None, f1_seed: int = 0,
+                   mesh_metrics: bool = False) -> dict:
     """Losses of one eval-mode output dict (keys ``vertex_positions`` (list, incl. the cubified stage-0 set), ``faces``,
     ``edge_index``, ``vertice_index``, ``face_index``; optional ``voxels``) against ``batch`` (``.meshes``,
     ``.vertice_index``, ``.face_index``, optional ``.voxels``) -- what reference ``validate`` computes per batch
@@ -127,7 +246,10 @@ def validate_batch(model_output: dict, batch, point_cloud_size: float = 10e3, nu
 
     Added (SURVEY 8 f-3): ``f1@tau`` of the final meshes -- precision = share of predicted surface samples within ``tau`` of
     the ground-truth samples, recall the converse, F1 = 2PR / (P + R) in percent, averaged over the meshes; it costs one
-    extra nearest-neighbour call (k = 0) on 10 000-point clouds of the normalised meshes."""
+    extra nearest-neighbour call (k = 0) on 10 000-point clouds of the normalised meshes.
+
+    ``mesh_metrics=True`` adds the ``compare_meshes`` keys of the final meshes (GT-10 scale, default thresholds, seed
+    ``f1_seed + 2``) and ``num_valid``; the default leaves the output as it was."""
     from . import functional as F_
     from .loss_functions import batched_mesh_loss, voxel_loss
     vs, fs, e_index = model_output["vertex_positions"], model_output["faces"], model_output["edge_index"]
@@ -148,6 +270,9 @@ def validate_batch(model_output: dict, batch, point_cloud_size: float = 10e3, nu
         prec = (d_p < tau).float().mean(dim=1)
         rec = (d_g < tau).float().mean(dim=1)
         out["f1@%g" % tau] = (100.0 * 2 * prec * rec / (prec + rec).clamp_min(1e-8)).mean()
+    if mesh_metrics:
+        out.update(compare_meshes(vs[-1], fs, v_index, f_index, gt_pos, gt_faces, batch.vertice_index, batch.face_index,
+                                  seed=f1_seed + 2))
     return out
 
 
@@ -167,17 +292,25 @@ class AverageMeter:
         return self.sum / max(self.count, 1)
 
 
-def validate(model, val_loader, device=None, point_cloud_size: float = 10e3, num_neighbours_for_normal_loss: int = 10) -> dict:
+def validate(model, val_loader, device=None, point_cloud_size: float = 10e3, num_neighbours_for_normal_loss: int = 10,
+             mesh_metrics: bool = False) -> dict:
     """Mesh-side validation loop (reference ``validate``, eval_utils.py:93-194, without the backbone / classification
     metrics that are outside the hot path): ``model(images)`` must return the eval-mode output dict; returns AverageMeters
-    named like the reference's (``voxel_loss``, ``chamfer_loss``, ``normal_loss``, ``edge_loss``) plus ``f1@tau``."""
+    named like the reference's (``voxel_loss``, ``chamfer_loss``, ``normal_loss``, ``edge_loss``) plus ``f1@tau``.
+    ``mesh_metrics=True`` adds the ``compare_meshes`` metrics of the final meshes, each batch weighted by its number of
+    valid (non-empty) predicted meshes."""
     model.eval()
     meters = {}
     for batch in val_loader:
         if device is not None:
             batch = batch.to(device, non_blocking=True)
-        res = validate_batch(model(batch.images), batch, point_cloud_size, num_neighbours_for_normal_loss)
+        res = validate_batch(model(batch.images), batch, point_cloud_size, num_neighbours_for_normal_loss,
+                             mesh_metrics=mesh_metrics)
         n = len(batch.vertice_index)
+        n_valid = res.pop("num_valid", None)
         for k, v in res.items():
-            meters.setdefault(k, AverageMeter(k)).update(float(v), n)
+            if k not in _PAPER_KEYS:
+                meters.setdefault(k, AverageMeter(k)).update(float(v), n)
+            elif n_valid:                        # a batch without a valid predicted mesh adds nothing to these means
+                meters.setdefault(k, AverageMeter(k)).update(float(v), n_valid)
     return meters

@@ -1255,6 +1255,84 @@ def sample_points(verts: Tensor, faces: Tensor, v_index: Sequence[int], f_index:
                          max(f_index) if B else 0, int(n), u, face_idx, xi2, xi1, seed, cdf)
 
 
+@torch.no_grad()
+def sample_surface(verts: Tensor, faces: Tensor, v_index: Sequence[int], f_index: Sequence[int], n: int,
+                   u: Optional[Tensor] = None, face_idx: Optional[Tensor] = None, xi2: Optional[Tensor] = None,
+                   xi1: Optional[Tensor] = None, seed: Optional[int] = None, cdf_owner=None,
+                   scale: Optional[Tensor] = None, v_starts: Optional[Sequence[int]] = None) -> Tuple[Tensor, Tensor, Tensor]:
+    """Eval-side surface sample (no autograd): ``(points B x n x 3, unit face normals B x n x 3, global face ids B x n)``.
+    The points are those of ``sample_points`` for the same randomness arguments before its unit-ball normalisation,
+    multiplied by ``scale[b]`` (optional per-mesh fp32 CUDA tensor, e.g. from ``mesh_gt_scale``).  ``v_starts``: first
+    vertex row of every mesh when the listed meshes are not the whole packed buffer (meshes without faces filtered out of
+    the lists); by default the running sum of ``v_index``."""
+    dev = verts.device
+    _require_cuda(verts, "sample_surface")
+    B = len(f_index)
+    if len(v_index) != B:
+        raise RuntimeError("sample_surface: v_index and f_index must have the same length")
+    if B and min(f_index) <= 0:
+        raise RuntimeError("sample_surface: every mesh needs at least one face")
+    if v_starts is None and (sum(v_index) != verts.shape[0] or sum(f_index) != faces.shape[0]):
+        raise RuntimeError("sample_surface: index lists do not match the packed tensors")
+    if seed is None:
+        seed = _next_seed() if xi2 is None else 0
+    n = int(n)
+    v = _f32c(verts.detach())
+    f = faces.contiguous().long()
+    f_off = offsets_table(f_index, dev)
+    v_off = offsets_table(v_index, dev) if v_starts is None else _device_table("off", list(v_starts) + [v.shape[0]], dev)
+    cdf = None
+    if face_idx is None and B:
+        cdf = (cached_face_cdf(cdf_owner, verts, faces, v_index, f_index) if cdf_owner is not None and v_starts is None
+               else _face_cdf(v, f, v_off, f_off, B, max(f_index)))
+    points = torch.empty(B, n, 3, dtype=torch.float32, device=dev)
+    normals = torch.empty(B, n, 3, dtype=torch.float32, device=dev)
+    fidx = torch.empty(B, n, dtype=torch.int32, device=dev)
+    cv = lambda t, dt: None if t is None else t.to(device=dev, dtype=dt).contiguous()
+    u, xi2, xi1, sc = cv(u, torch.float32), cv(xi2, torch.float32), cv(xi1, torch.float32), cv(scale, torch.float32)
+    face_idx = cv(face_idx, torch.int64)
+    _lib.call("mrb_sample_surface_fwd", _lib.ptr(v), _lib.ptr(f), _lib.ptr(v_off), _lib.ptr(f_off), _lib.ptr(cdf), B, n,
+              _lib.ptr(u), _lib.ptr(face_idx), _lib.ptr(xi2), _lib.ptr(xi1), int(seed), _lib.ptr(sc), _lib.ptr(points),
+              _lib.ptr(normals), _lib.ptr(fidx))
+    return points, normals, fidx
+
+
+@torch.no_grad()
+def mesh_gt_scale(verts: Tensor, v_index: Sequence[int], target: float = 10.0) -> Tensor:
+    """fp32 [B]: ``target / longest side of the bounding box`` of every mesh of a packed vertex buffer (the paper's GT-10
+    normalisation with ``target = 10``).  A mesh of zero extent gets inf."""
+    _require_cuda(verts, "mesh_gt_scale")
+    dev = verts.device
+    v = _f32c(verts.detach())
+    if sum(v_index) != v.shape[0]:
+        raise RuntimeError("mesh_gt_scale: v_index does not match the packed vertices")
+    scale = torch.empty(len(v_index), dtype=torch.float32, device=dev)
+    _lib.call("mrb_mesh_gt_scale", _lib.ptr(v), _lib.ptr(offsets_table(v_index, dev)), len(v_index), float(target),
+              _lib.ptr(scale))
+    return scale
+
+
+MAX_THRESHOLDS = 8
+
+
+@torch.no_grad()
+def mesh_metrics(d_p: Tensor, i_p: Tensor, d_q: Tensor, i_q: Tensor, n_p: Tensor, n_q: Tensor,
+                 thresholds: Sequence[float]) -> Tensor:
+    """fp32 [B, 3 + 3T] per-mesh metrics from the k = 0 outputs of ``knn_search`` and the sample normals: Chamfer-L2,
+    NormalConsistency, AbsNormalConsistency, then (Precision, Recall, F1) in percent for every threshold (T <= 8)."""
+    _require_cuda(d_p, "mesh_metrics")
+    thr = [float(t) for t in thresholds]
+    if len(thr) > MAX_THRESHOLDS:
+        raise ValueError("mesh_metrics: at most %d thresholds, got %d" % (MAX_THRESHOLDS, len(thr)))
+    B, P = d_p.shape
+    Q = d_q.shape[1]
+    out = torch.empty(B, 3 + 3 * len(thr), dtype=torch.float32, device=d_p.device)
+    taus = (ctypes.c_float * max(1, len(thr)))(*thr)
+    _lib.call("mrb_mesh_metrics", _lib.ptr(d_p), _lib.ptr(i_p), _lib.ptr(d_q), _lib.ptr(i_q), _lib.ptr(_f32c(n_p)),
+              _lib.ptr(_f32c(n_q)), B, P, Q, ctypes.addressof(taus), len(thr), _lib.ptr(out))
+    return out
+
+
 KNN_ALGOS = {"auto": 0, "tiled": 1, "grid": 2}
 
 

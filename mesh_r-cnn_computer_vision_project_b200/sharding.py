@@ -222,6 +222,22 @@ def all_reduce_losses(losses: dict) -> dict:
     return {k: buf[i] for i, k in enumerate(keys)}
 
 
+def reduce_mesh_metrics(per_mesh: dict) -> dict:
+    """Means of the per-mesh metrics of ``eval_utils.compare_meshes(..., reduce=False)`` over the valid meshes of ALL ranks,
+    plus ``num_valid`` (int): one all-reduce(SUM) of the per-key sums and the count, so that evaluation with one process per
+    GPU does not average per-rank means.  Without a process group (or at world size 1) the same means over the local
+    meshes.  The input is not modified."""
+    from .eval_utils import mesh_metric_sums
+    keys, buf = mesh_metric_sums(per_mesh)
+    if _dist_on():
+        dist.all_reduce(buf, op=dist.ReduceOp.SUM)
+    count = int(buf[-1])
+    means = (buf[:-1] / count).float() if count else torch.full((len(keys),), float("nan"), device=buf.device)
+    out = {k: means[i] for i, k in enumerate(keys)}
+    out["num_valid"] = count
+    return out
+
+
 def _all_gather_ragged(t: Tensor, dim: int = 0) -> List[Tensor]:
     """all_gather of tensors whose size along ``dim`` differs per rank (sizes exchanged first, payload padded to the max)."""
     world = dist.get_world_size()
