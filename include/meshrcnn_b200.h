@@ -294,7 +294,13 @@ int mrb_chamfer_bwd(const float* a, const float* b, int B, int P, int Q, const i
  * reference meshRCNN/loss_functions.py:107-170,175-189 (incl. the S.cpu() -> symeig -> .to(device) round trip).
  *   mrb_normals_fwd     normal[b,p] = row 0 of the (ascending, canonically signed) eigenvector matrix of the 3x3
  *                       scatter matrix of pt[b, knn[b,p,:]]
- *   mrb_normals_bwd     gn -> gpt (atomic accumulate into B x P x 3)
+ *   mrb_normals_bwd     gn -> gpt (atomic accumulate into B x P x 3); rows with gn = 0 are skipped.  Degenerate spectra: the
+ *                       derivative of an eigenvector divides by the gap to each other eigenvalue, and a pair of eigenvalues
+ *                       closer than 1e-14 * (|w0| + |w1| + |w2|) contributes nothing instead.  So a row whose three eigenvalues
+ *                       coincide (k = 1, all k neighbours the same point, an isotropic neighbourhood) has an exactly zero
+ *                       gradient, and a row with one coinciding pair (k = 2, a square axis-aligned planar patch) keeps only the
+ *                       terms of the other pairs; both stay finite.  The forward normal of such a row is unit length, but
+ *                       within the degenerate eigenspace its direction is the eigensolver's choice, not a defined quantity.
  *   mrb_normals_fwd_eig also writes the eigen-decomposition: eig = 12 planes of B * P doubles (w0 w1 w2 | V row-major)
  *   mrb_normals_bwd_ld  the same into rows of ld_gpt floats: 3, or 4 (xyz + one unused lane, 16-byte aligned) -- the padded
  *                       layout turns the 3 scalar atomics per neighbour into one 16-byte vector reduction; eig (may be

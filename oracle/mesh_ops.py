@@ -155,13 +155,18 @@ def normalize_cloud(pts: Tensor) -> Tensor:
     return c / torch.sqrt((c * c).sum(1).max())
 
 
-def sample_with(verts: Tensor, faces: Tensor, face_idx: Tensor, xi2: Tensor, xi1: Tensor) -> Tensor:
+def sample_raw_with(verts: Tensor, faces: Tensor, face_idx: Tensor, xi2: Tensor, xi1: Tensor) -> Tensor:
     """mesh_sampling.py:18-35 with the three random draws injected: ``face_idx`` (= multinomial, :16),
-    ``xi2`` (= first rand, :20), ``xi1`` (= second rand, before the sqrt, :21)."""
+    ``xi2`` (= first rand, :20), ``xi1`` (= second rand, before the sqrt, :21); the points before normalisation."""
     tri = verts[faces[face_idx]]                       # n x 3 x 3
     r = xi1.sqrt()
     w = torch.stack([1.0 - r, (1 - xi2) * r, xi2 * r], dim=1).to(verts.dtype)
-    return normalize_cloud((tri * w.unsqueeze(2)).sum(1))
+    return (tri * w.unsqueeze(2)).sum(1)
+
+
+def sample_with(verts: Tensor, faces: Tensor, face_idx: Tensor, xi2: Tensor, xi1: Tensor) -> Tensor:
+    """``sample_raw_with`` normalised into the unit ball (mesh_sampling.py:6-35)."""
+    return normalize_cloud(sample_raw_with(verts, faces, face_idx, xi2, xi1))
 
 
 def face_cdf_draw(verts: Tensor, faces: Tensor, u: Tensor) -> Tensor:
@@ -269,6 +274,67 @@ def normal_distance(p: Tensor, q: Tensor, d: Tensor, idx_p: Tensor, idx_q: Tenso
     l0 = (n_p * n_q[ar, idx_p]).sum(2).abs().sum()
     l1 = (n_q * n_p[ar, idx_q]).sum(2).abs().sum()
     return l0, l1
+
+
+# ----------------------------------------------------------------------------------------------------------
+# the same losses with the discrete choices given (face draws, nearest indices, k-NN sets): O(n) memory, so the
+# continuous part can be differentiated in fp64 at the trained shape (B = 32, 10 000 points) where the dense
+# B x P x Q matrices above would not fit
+# ----------------------------------------------------------------------------------------------------------
+def chamfer_given(p: Tensor, q: Tensor, idx_p: Tensor, idx_q: Tensor):
+    """(sum_i |p_i - q_{idx_p[i]}|^2, sum_j |q_j - p_{idx_q[j]}|^2) for B x P x 3 / B x Q x 3 clouds: ``chamfer`` of the
+    dense matrix when idx_* are its argmins (loss_functions.py:93-102)."""
+    ar = torch.arange(p.shape[0]).view(-1, 1)
+    return ((p - q[ar, idx_p.long()]) ** 2).sum(), ((q - p[ar, idx_q.long()]) ** 2).sum()
+
+
+def normal_sums_given(p: Tensor, q: Tensor, knn_p: Tensor, knn_q: Tensor, idx_p: Tensor, idx_q: Tensor,
+                      canonical_signs: bool = True):
+    """``normal_distance`` (loss_functions.py:107-126) with the k-NN sets and nearest indices given."""
+    n_p = normals_from_neighbours(p, knn_p.long(), canonical_signs)
+    n_q = normals_from_neighbours(q, knn_q.long(), canonical_signs)
+    ar = torch.arange(p.shape[0]).view(-1, 1)
+    return (n_p * n_q[ar, idx_p.long()]).sum(2).abs().sum(), (n_q * n_p[ar, idx_q.long()]).sum(2).abs().sum()
+
+
+def normal_total_given(p: Tensor, q: Tensor, knn_p: Tensor, knn_q: Tensor, idx_p: Tensor, idx_q: Tensor, scale: float,
+                       canonical_signs: bool = True) -> Tensor:
+    """scale * (sum of both normal-consistency sums) -- loss_functions.py:69-72 with scale = -1 / point_cloud_size."""
+    l0, l1 = normal_sums_given(p, q, knn_p, knn_q, idx_p, idx_q, canonical_signs)
+    return scale * (l0 + l1)
+
+
+def normals_conditioning(pt: Tensor, nn_idx: Tensor):
+    """How far each row of ``normals_from_neighbours`` is from a discontinuity, in fp64, as four B x P tensors:
+    (gap, m_v20, m_col1, m_det).  gap = min_{i != j} |w_i - w_j| / w_2 is the smallest relative eigen-gap (the
+    eigenvector derivative divides by it; 0 for a degenerate spectrum).  The other three are the margins of the
+    canonical sign rules (``canonical_eigvec_signs``): |V[2,0]|, the difference of the two largest |.| of column 1, and
+    |det V|.  A row whose gap or margin is at the level of the rounding of its inputs may legitimately differ between
+    two correct implementations."""
+    pt = pt.detach().double()
+    B, P, _ = pt.shape
+    nb = pt[torch.arange(B).view(-1, 1, 1), nn_idx.long()]
+    y = nb - nb.mean(2, keepdim=True)
+    w, v = torch.linalg.eigh(y.transpose(-2, -1) @ y, UPLO="U")
+    top = w[..., 2].abs().clamp_min(1e-300)
+    gap = torch.stack([w[..., 1] - w[..., 0], w[..., 2] - w[..., 1]], -1).abs().min(-1).values / top
+    c1 = v[..., :, 1].abs().sort(-1, descending=True).values
+    return gap, v[..., 2, 0].abs(), c1[..., 0] - c1[..., 1], torch.linalg.det(v).abs()
+
+
+def nearest_chunked(p: Tensor, q: Tensor, rows: int = 1024) -> Tensor:
+    """B x P fp64 squared distance from every p_i to its nearest q_j, in row chunks of ``rows`` (memory rows x Q per
+    cloud instead of P x Q for the whole batch).  |p|^2 + |q|^2 - 2 p.q in fp64: for fp32 clouds of unit scale the
+    cancellation error (~1e-15) is far below the fp32 resolution the callers compare at."""
+    p, q = p.detach().double(), q.detach().double()
+    out = torch.empty(p.shape[:2], dtype=torch.float64)
+    rq = (q * q).sum(2)
+    for b in range(p.shape[0]):
+        for s in range(0, p.shape[1], rows):
+            a = p[b, s:s + rows]
+            d = (a * a).sum(1, keepdim=True) + rq[b].unsqueeze(0) - 2.0 * (a @ q[b].t())
+            out[b, s:s + rows] = d.min(1).values.clamp_min(0.0)
+    return out
 
 
 def mesh_loss_with(pos, faces, adj, v_index, f_index, gt_pos, gt_faces, gt_v_index, gt_f_index,

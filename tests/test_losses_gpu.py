@@ -119,14 +119,22 @@ def test_knn_ragged_sizes_vs_oracle(lib, B, P, Q, k):
     from meshrcnn_b200 import functional as F_
     gen = torch.Generator().manual_seed(B * 1000 + P)
     p, q = torch.rand(B, P, 3, generator=gen) - 0.5, torch.rand(B, Q, 3, generator=gen) - 0.5
-    l1, l2, ip, iq, kp, kq = F_.chamfer_knn(p.cuda(), q.cuda(), k)
+    pc, qc = p.cuda().requires_grad_(), q.cuda().requires_grad_()
+    l1, l2, ip, iq, kp, kq = F_.chamfer_knn(pc, qc, k)
     _, ip_t, kp_t, _, iq_t, kq_t = F_.knn_search(p.cuda(), q.cuda(), k, algo="tiled")
     assert torch.equal(ip, ip_t) and torch.equal(iq, iq_t) and (not k or (torch.equal(kp, kp_t) and torch.equal(kq, kq_t)))
-    d = mesh_ops.p2p_distance(p.double(), q.double())
+    p64, q64 = p.double().requires_grad_(), q.double().requires_grad_()
+    d = mesh_ops.p2p_distance(p64, q64)
     w1, wi1, w2, wi2 = mesh_ops.chamfer(d)
-    close(l1, w1, what="l1")
-    close(l2, w2, what="l2")
+    close(l1, w1.detach(), what="l1")
+    close(l2, w2.detach(), what="l2")
     assert torch.equal(ip.cpu().long(), wi1) and torch.equal(iq.cpu().long(), wi2)
+    # gradients of both sums through the dense fp64 matrix (P != Q: the two scatter directions must not be swapped)
+    gp, gq = torch.autograd.grad(0.7 * l1 + 1.3 * l2, [pc, qc])
+    hp, hq = torch.autograd.grad(0.7 * w1 + 1.3 * w2, [p64, q64])
+    close(gp, hp, what="grad p")
+    close(gq, hq, what="grad q")
+    d = d.detach()
     if k:
         for got, dd in ((kp, d), (kq, d.transpose(1, 2))):
             want = dd.topk(k, dim=2, largest=False).indices.sort(-1).values
