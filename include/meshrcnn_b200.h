@@ -212,6 +212,31 @@ int mrb_vert_align_proj_bwd(const float* gout, int ld_g, int D, int n_maps, cons
                             const float* pos, const int32_t* vert_mesh, const int32_t* mesh_info, int SV, float* gT,
                             void* stream);
 
+/* Bilinear VertexAlign (opt-in mode; csrc/vert_align_bilinear.cu), differentiable in the vertex positions.  One square S x S
+ * map given as channels-last fp32 rows: texel (i, j) of image img is rows[((img * S + i) * S + j) * ld_rows + 0 .. D-1] (the
+ * output of mrb_feature_map_to_rows, or per-texel projections T of it).  Projection as mrb_vert_align_fwd up to and including
+ * the clamps to the image (x = w / sx indexes the H axis, y = h / sy the W axis), then x, y clamped to [0, S-1] and
+ *   out[v] = (1-fx)(1-fy) f[x0,y0] + (1-fx) fy f[x0,y0+1] + fx (1-fy) f[x0+1,y0] + fx fy f[x0+1,y0+1]
+ * with x0 = clamp(floor(x), 0, S-2), fx = x - x0 (y0, fy alike); S == 1 gives f[0,0].  This is grid_sample(align_corners=True,
+ * padding_mode="border") at (x, y).
+ *   mrb_vert_align_bilinear_fwd  out[v, 0:D] = sample (accumulate == 0) or += sample (accumulate != 0); out rows of pitch
+ *                                ld_out (pass a column-offset pointer to fill a column block)
+ *   mrb_vert_align_bilinear_bwd  grows (may be NULL; zero-filled by the caller, pitch ld_grows) += w_corner * gout[v] for the
+ *                                four corners (fp32 reductions); gpos (may be NULL, SV x 3) = (accumulate_gpos == 0) or +=
+ *                                (!= 0) the position gradient, written by the one warp that owns the vertex (no atomics:
+ *                                deterministic, and calls for several maps issued in sequence on one stream may accumulate).
+ *                                Clamps pass the gradient inside their closed interval; at a texel knot the derivative is the
+ *                                one-sided one of the cell the floor rule picks; where the projection or its derivative is not
+ *                                finite (p2 == 0, NaN positions) the sample is the clamped one and the gradient is exactly 0.
+ * Every mesh_info image index must be < n_img (the caller validates; the kernels clamp it as well).  SV == 0 returns 0
+ * without a launch; D, S, n_img >= 1 and pitches >= D are required.  float4 path when D % 4 == 0 and all rows 16-byte aligned. */
+int mrb_vert_align_bilinear_fwd(const float* rows, int ld_rows, int D, int S, int n_img, const float* pos,
+                                const int32_t* vert_mesh, const int32_t* mesh_info, int SV, int accumulate, float* out,
+                                int ld_out, void* stream);
+int mrb_vert_align_bilinear_bwd(const float* gout, int ld_g, const float* rows, int ld_rows, int D, int S, int n_img,
+                                const float* pos, const int32_t* vert_mesh, const int32_t* mesh_info, int SV, float* grows,
+                                int ld_grows, float* gpos, int accumulate_gpos, void* stream);
+
 /* ------------------------------------------------------------------------------------------------------------
  * Surface sampling -- replaces utils/mesh_sampling.py:6-57 (sample, surface_areas), utils/process.py:7-20
  * (normalize_mesh) and the per-mesh loop of batched_mesh_sampling (meshRCNN/loss_functions.py:80-89).

@@ -133,7 +133,7 @@ LAUNCHES = {
     "mrb_cubify_count": 4, "mrb_cubify_emit": 3, "mrb_coo_to_csr": 5, "mrb_csr_gather_fwd": 1, "mrb_relu_mask": 1, "mrb_graphconv_bwd_gather": 1,
     "mrb_segment_ids": 1, "mrb_sgemm": 1, "mrb_gemm_tc": 1, "mrb_gemm_tc_pack": 1, "mrb_gemm_tc_pack_graphconv": 1, "mrb_gemm_tc_pack_graphconv_batch": 1, "mrb_gemm_tc_wgrad": 1, "mrb_vert_align_fwd": 2, "mrb_vert_align_bwd": 1,
     "mrb_vert_align_fwd_bf16": 2, "mrb_feature_map_to_rows": 1, "mrb_rows_to_feature_map": 1, "mrb_vert_align_proj_fwd": 1,
-    "mrb_vert_align_proj_bwd": 1, "mrb_gemm_tc_acc": 1, "mrb_gemm_tc_wgrad_split": 1, "mrb_vert_align_texrows": 1,
+    "mrb_vert_align_proj_bwd": 1, "mrb_vert_align_bilinear_fwd": 1, "mrb_vert_align_bilinear_bwd": 1, "mrb_gemm_tc_acc": 1, "mrb_gemm_tc_wgrad_split": 1, "mrb_vert_align_texrows": 1,
     "mrb_gc_gather_fwd": 1, "mrb_gc_gather_bwd": 1, "mrb_head_fwd": 1, "mrb_head_bwd": 1, "mrb_voxel_bce_fwd": 2, "mrb_voxel_bce_bwd": 1, "mrb_normal_loss_total_fwd": 2,
     "mrb_normal_loss_total_bwd": 1, "mrb_scalar_combine": 1, "mrb_scalar_scatter": 1, "mrb_face_areas": 1,
     "mrb_face_area_cdf": 2, "mrb_sample_points_fwd": 2, "mrb_normalize_cloud_fwd": 1, "mrb_sample_points_bwd": 2, "mrb_sample_points_bwd_ld": 2,

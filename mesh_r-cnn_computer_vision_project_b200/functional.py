@@ -987,6 +987,184 @@ def vert_align(img_features: Sequence[Tensor], vertex_positions: Tensor, vertice
     return _VertAlign.apply(vertex_positions, vert_mesh, info, *img_features)
 
 
+# ----------------------------------------------------------------------------------------------------------
+# bilinear VertexAlign (opt-in; csrc/vert_align_bilinear.cu): differentiable in the vertex positions
+# ----------------------------------------------------------------------------------------------------------
+def _square_maps(fmaps: Sequence[Tensor], what: str) -> List[Tensor]:
+    maps = []
+    for f in fmaps:
+        _require_cuda(f, what)
+        if f.dim() != 4 or f.shape[2] != f.shape[3]:
+            raise RuntimeError("VertexAlign: feature maps must be N x C x H x W with H == W (the reference indexes H with the "
+                               "x coordinate)")
+        maps.append(_map_tensor(f))
+    return maps
+
+
+def _bilinear_tables(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
+                     mesh_index: Sequence[int], image_sizes):
+    """(vert_mesh, mesh_info) of the bilinear kernels after the host-side checks that keep every index they read in range:
+    each vertex's mesh has a mesh_info row, and each image that holds a mesh exists in every map.  vert_mesh is built from
+    ``vertices_per_mesh`` itself (not taken from a registered topology), so it cannot name a mesh the table lacks."""
+    _require_cuda(vertex_positions, "VertexAlign")
+    if vertex_positions.dim() != 2 or vertex_positions.shape[1] != 3:
+        raise RuntimeError("VertexAlign: vertex positions must be SV x 3")
+    if len(mesh_index) != len(image_sizes):
+        raise RuntimeError("VertexAlign: mesh_index and image_sizes differ in length")
+    if any(int(m) < 0 for m in mesh_index) or any(int(c) < 0 for c in vertices_per_mesh):
+        raise RuntimeError("VertexAlign: negative mesh or vertex count")
+    if sum(int(m) for m in mesh_index) != len(vertices_per_mesh):
+        raise RuntimeError("VertexAlign: sum(mesh_index) must equal the number of meshes")
+    if sum(int(c) for c in vertices_per_mesh) != vertex_positions.shape[0]:
+        raise RuntimeError("VertexAlign: vertices_per_mesh does not sum to the number of vertex positions")
+    used = [i for i, m in enumerate(mesh_index) if int(m) > 0]
+    for f in img_features:
+        if used and f.dim() == 4 and used[-1] >= f.shape[0]:
+            raise RuntimeError("VertexAlign: image %d holds a mesh but the feature map has %d images" % (used[-1], f.shape[0]))
+    dev = vertex_positions.device
+    SV = vertex_positions.shape[0]
+    vert_mesh = vertex_mesh_ids(vertices_per_mesh, SV, dev) if SV else torch.empty(0, dtype=torch.int32, device=dev)
+    return vert_mesh, mesh_info_table(mesh_index, image_sizes, dev)
+
+
+class _VertAlignBilinear(torch.autograd.Function):
+    """Bilinear VertexAlign of every map into its column block of an SV x sum(C_m) output; gradients to the maps and to the
+    vertex positions (csrc/vert_align_bilinear.cu)."""
+
+    @staticmethod
+    def forward(ctx, pos, vert_mesh, mesh_info, *fmaps):
+        pos_c = _f32c(pos.detach())
+        maps = _square_maps(fmaps, "VertexAlign")
+        SV = pos_c.shape[0]
+        ctot = sum(m.shape[1] for m in maps)
+        out = torch.empty(SV, ctot, dtype=torch.float32, device=pos.device)
+        rows, off = [], 0
+        for m in maps:
+            n_img, C, S, _ = m.shape
+            r = feature_rows(m)
+            _lib.call("mrb_vert_align_bilinear_fwd", _lib.ptr(r), C, C, S, n_img, _lib.ptr(pos_c), _lib.ptr(vert_mesh),
+                      _lib.ptr(mesh_info), SV, 0, _lib.ptr(out) + 4 * off, ctot)
+            rows.append(r)
+            off += C
+        ctx.save_for_backward(pos_c, vert_mesh, mesh_info, *rows)
+        ctx.shapes = [tuple(m.shape) for m in maps]
+        ctx.dtypes = [f.dtype for f in fmaps]
+        ctx.pos_dtype = pos.dtype
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        pos_c, vert_mesh, mesh_info = ctx.saved_tensors[:3]
+        rows = ctx.saved_tensors[3:]
+        gout = _rows(gout)
+        SV, ldg = gout.shape[0], gout.stride(0)
+        dev = gout.device
+        gpos = torch.zeros(SV, 3, dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
+        grads, off = [], 0
+        for i, (shape, r) in enumerate(zip(ctx.shapes, rows)):
+            n_img, C, S, _ = shape
+            grows = torch.zeros(r.shape, dtype=torch.float32, device=dev) if ctx.needs_input_grad[3 + i] else None
+            if grows is not None or gpos is not None:
+                _lib.call("mrb_vert_align_bilinear_bwd", gout.data_ptr() + 4 * off, ldg, _lib.ptr(r), C, C, S, n_img,
+                          _lib.ptr(pos_c), _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, _lib.ptr(grows), C, _lib.ptr(gpos), 1)
+            if grows is not None:
+                g = torch.empty(shape, dtype=torch.float32, device=dev)
+                _lib.call("mrb_rows_to_feature_map", _lib.ptr(grows), C, n_img, C, S * S, _lib.ptr(g))
+                grads.append(g if ctx.dtypes[i] == torch.float32 else g.to(ctx.dtypes[i]))
+            else:
+                grads.append(None)
+            off += C
+        if gpos is not None and ctx.pos_dtype != torch.float32:
+            gpos = gpos.to(ctx.pos_dtype)
+        return (gpos, None, None) + tuple(grads)
+
+
+def vert_align_bilinear(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
+                        image_sizes, mesh_index: Sequence[int]) -> Tensor:
+    """Bilinear VertexAlign (the opt-in mode of ``layers.VertexAlign``): SV x sum(C_m), differentiable in every map and in
+    ``vertex_positions``.  Same projection and axis convention as ``vert_align``; each square map is then sampled like
+    ``grid_sample(align_corners=True, padding_mode="border")`` -- see csrc/vert_align_bilinear.cu for the exact
+    definition.  fp32 or bf16 maps; the output and the position gradient are fp32, map gradients come in the map's dtype."""
+    vert_mesh, info = _bilinear_tables(img_features, vertex_positions, vertices_per_mesh, mesh_index, image_sizes)
+    return _VertAlignBilinear.apply(vertex_positions, vert_mesh, info, *img_features)
+
+
+def _project_texels(maps: Sequence[Tensor], w: Tensor, n_img: int):
+    """T = per-texel projections of every map, packed map after map: T[r0_m + r] = rows_m[r] @ W[:, c0_m:c0_m+C_m]^T, with
+    rows_m the channels-last fp32 rows of map m in (image, x1, y1) order.  Returns (T, [rows_m], [R_m])."""
+    lib = _lib.load()
+    dev = w.device
+    D, ctot = w.shape
+    rows_per_map = [n_img * m.shape[2] * m.shape[3] for m in maps]
+    T = torch.empty(sum(rows_per_map), D, dtype=torch.float32, device=dev)
+    rows_cl, r0, c0 = [], 0, 0
+    for m, R in zip(maps, rows_per_map):
+        C = m.shape[1]
+        cl = torch.empty(R, C, dtype=torch.float32, device=dev)
+        _lib.call("mrb_feature_map_to_rows", _lib.ptr(m), int(m.dtype == torch.bfloat16), n_img, C, R // n_img, _lib.ptr(cl))
+        # T[r0:r0+R] = cl @ W[:, c0:c0+C]^T : logical operand B(k, n) = W[n, c0 + k]
+        if _use_tc(C, D):
+            img = torch.empty(lib.mrb_gemm_tc_image_bytes(C, D), dtype=torch.uint8, device=dev)
+            _lib.call("mrb_gemm_tc_pack", w.data_ptr() + 4 * c0, None, 1, ctot, 0, 0, C, D, _lib.ptr(img))
+            tc_gemm(_lib.ptr(cl), C, R, C, img, D, T.data_ptr() + 4 * r0 * D, D)
+        else:
+            _gemm(False, True, R, D, C, _lib.ptr(cl), C, w.data_ptr() + 4 * c0, ctot, 0.0, T.data_ptr() + 4 * r0 * D, D)
+        rows_cl.append(cl)
+        r0 += R
+        c0 += C
+    return T, rows_cl, rows_per_map
+
+
+def _backproject_texels(gT: Tensor, w: Tensor, rows_cl, shapes, rows_per_map, dtypes, n_img: int, want_w: bool, want_maps):
+    """Weight and map gradients from the gradient gT of the packed projections T (``_project_texels``): dW_m^T = rows_m^T @
+    gT_m and d map_m = NCHW(gT_m @ W[:, c0_m:c0_m+C_m]).  Returns (gW or None, [gmap_m or None])."""
+    lib = _lib.load()
+    dev = gT.device
+    D, ctot = w.shape
+    gwt = torch.zeros(ctot, D, dtype=torch.float32, device=dev) if want_w else None
+    gmaps = []
+    r0 = c0 = 0
+    for i, (shape, R, cl) in enumerate(zip(shapes, rows_per_map, rows_cl)):
+        C = shape[1]
+        gt_ptr = gT.data_ptr() + 4 * r0 * D
+        if gwt is not None:             # dW_m^T (C x D) = rows_m^T @ gT_m
+            if _use_tc_wgrad(R, D):
+                _lib.call("mrb_gemm_tc_wgrad", _lib.ptr(cl), C, gt_ptr, D, R, C, D, gwt.data_ptr() + 4 * c0 * D, None, D, D)
+            else:
+                _gemm(True, False, C, D, R, _lib.ptr(cl), C, gt_ptr, D, 0.0, gwt.data_ptr() + 4 * c0 * D, D)
+        if want_maps[i]:                # d rows_m (R x C) = gT_m @ W[:, c0:c0+C] : B(k, n) = W[k, c0 + n]
+            g_rows = torch.empty(R, C, dtype=torch.float32, device=dev)
+            if _use_tc(D, C):
+                img = torch.empty(lib.mrb_gemm_tc_image_bytes(D, C), dtype=torch.uint8, device=dev)
+                _lib.call("mrb_gemm_tc_pack", w.data_ptr() + 4 * c0, None, ctot, 1, 0, 0, D, C, _lib.ptr(img))
+                tc_gemm(gt_ptr, D, R, D, img, C, _lib.ptr(g_rows), C)
+            else:
+                _gemm(False, False, R, C, D, gt_ptr, D, w.data_ptr() + 4 * c0, ctot, 0.0, _lib.ptr(g_rows), C)
+            g = torch.empty(shape, dtype=torch.float32, device=dev)
+            _lib.call("mrb_rows_to_feature_map", _lib.ptr(g_rows), C, n_img, C, R // n_img, _lib.ptr(g))
+            gmaps.append(g if dtypes[i] == torch.float32 else g.to(dtypes[i]))
+        else:
+            gmaps.append(None)
+        r0 += R
+        c0 += C
+    gw = gwt.t().contiguous() if gwt is not None else None      # nn.Linear stores out x in
+    return gw, gmaps
+
+
+def _linear_maps(weight: Tensor, fmaps: Sequence[Tensor]):
+    """(fp32 weight, maps, n_img) of linear(VertexAlign(maps)) after the shape checks."""
+    w = _f32c(weight)
+    D, ctot = w.shape
+    maps = _square_maps(fmaps, "VertexAlign+linear")
+    n_img = maps[0].shape[0]
+    if any(m.shape[0] != n_img for m in maps) or sum(m.shape[1] for m in maps) != ctot:
+        raise RuntimeError("VertexAlign+linear: maps %s do not match the %d x %d weight" %
+                           ([tuple(m.shape) for m in maps], D, ctot))
+    if D % 4 or not 1 <= len(maps) <= 8:
+        raise RuntimeError("VertexAlign+linear: out_features %% 4 == 0 and 1..8 maps required")
+    return w, maps, n_img
+
+
 class _VertAlignLinear(torch.autograd.Function):
     """linear(VertexAlign(maps))  =  sum over maps of  mask * (texel rows @ W_m^T)[texel(v)]   (csrc/align_proj.cu).
 
@@ -997,42 +1175,12 @@ class _VertAlignLinear(torch.autograd.Function):
     @staticmethod
     def forward(ctx, pos, vert_mesh, mesh_info, weight, *fmaps):
         _require_cuda(pos, "VertexAlign+linear")
-        lib = _lib.load()
         dev = pos.device
         pos_c = _f32c(pos.detach())
-        w = _f32c(weight)
-        D, ctot = w.shape
-        maps = []
-        for f in fmaps:
-            _require_cuda(f, "VertexAlign+linear")
-            if f.dim() != 4 or f.shape[2] != f.shape[3]:
-                raise RuntimeError("VertexAlign: feature maps must be N x C x H x W with H == W (the reference indexes H "
-                                   "with the x coordinate)")
-            maps.append(_map_tensor(f))
-        n_img = maps[0].shape[0]
-        if any(m.shape[0] != n_img for m in maps) or sum(m.shape[1] for m in maps) != ctot:
-            raise RuntimeError("VertexAlign+linear: maps %s do not match the %d x %d weight" %
-                               ([tuple(m.shape) for m in maps], D, ctot))
-        if D % 4 or not 1 <= len(maps) <= 8:
-            raise RuntimeError("VertexAlign+linear: out_features %% 4 == 0 and 1..8 maps required")
+        w, maps, n_img = _linear_maps(weight, fmaps)
+        D = w.shape[0]
         sizes = (ctypes.c_int * len(maps))(*[int(m.shape[2]) for m in maps])
-        rows_per_map = [n_img * m.shape[2] * m.shape[3] for m in maps]
-        T = torch.empty(sum(rows_per_map), D, dtype=torch.float32, device=dev)
-        rows_cl, r0, c0 = [], 0, 0
-        for m, R in zip(maps, rows_per_map):
-            C = m.shape[1]
-            cl = torch.empty(R, C, dtype=torch.float32, device=dev)
-            _lib.call("mrb_feature_map_to_rows", _lib.ptr(m), int(m.dtype == torch.bfloat16), n_img, C, R // n_img, _lib.ptr(cl))
-            # T[r0:r0+R] = cl @ W[:, c0:c0+C]^T : logical operand B(k, n) = W[n, c0 + k]
-            if _use_tc(C, D):
-                img = torch.empty(lib.mrb_gemm_tc_image_bytes(C, D), dtype=torch.uint8, device=dev)
-                _lib.call("mrb_gemm_tc_pack", w.data_ptr() + 4 * c0, None, 1, ctot, 0, 0, C, D, _lib.ptr(img))
-                tc_gemm(_lib.ptr(cl), C, R, C, img, D, T.data_ptr() + 4 * r0 * D, D)
-            else:
-                _gemm(False, True, R, D, C, _lib.ptr(cl), C, w.data_ptr() + 4 * c0, ctot, 0.0, T.data_ptr() + 4 * r0 * D, D)
-            rows_cl.append(cl)
-            r0 += R
-            c0 += C
+        T, rows_cl, rows_per_map = _project_texels(maps, w, n_img)
         SV = pos_c.shape[0]
         out = torch.empty(SV, D, dtype=torch.float32, device=dev)
         _lib.call("mrb_vert_align_proj_fwd", _lib.ptr(T), D, len(maps), sizes, n_img, _lib.ptr(pos_c), _lib.ptr(vert_mesh),
@@ -1046,50 +1194,79 @@ class _VertAlignLinear(torch.autograd.Function):
         pos_c, vert_mesh, mesh_info, w = ctx.saved_tensors[:4]
         rows_cl = ctx.saved_tensors[4:]
         sizes, n_img, shapes, dtypes, rows_per_map = ctx.meta
-        lib = _lib.load()
         dev = gout.device
-        D, ctot = w.shape
+        D = w.shape[0]
         gout = _rows(gout)
         SV = gout.shape[0]
         gT = torch.empty(sum(rows_per_map), D, dtype=torch.float32, device=dev)
         _lib.call("mrb_vert_align_proj_bwd", gout.data_ptr(), gout.stride(0), D, len(shapes), sizes, n_img, _lib.ptr(pos_c),
                   _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, _lib.ptr(gT))
-        gw = None
-        gwt = torch.zeros(ctot, D, dtype=torch.float32, device=dev) if ctx.needs_input_grad[3] else None
-        gmaps = []
-        r0 = c0 = 0
-        for i, (shape, R, cl) in enumerate(zip(shapes, rows_per_map, rows_cl)):
-            C = shape[1]
-            gt_ptr = gT.data_ptr() + 4 * r0 * D
-            if gwt is not None:             # dW_m^T (C x D) = rows_m^T @ gT_m
-                if _use_tc_wgrad(R, D):
-                    _lib.call("mrb_gemm_tc_wgrad", _lib.ptr(cl), C, gt_ptr, D, R, C, D, gwt.data_ptr() + 4 * c0 * D, None, D, D)
-                else:
-                    _gemm(True, False, C, D, R, _lib.ptr(cl), C, gt_ptr, D, 0.0, gwt.data_ptr() + 4 * c0 * D, D)
-            if ctx.needs_input_grad[4 + i]:  # d rows_m (R x C) = gT_m @ W[:, c0:c0+C] : B(k, n) = W[k, c0 + n]
-                g_rows = torch.empty(R, C, dtype=torch.float32, device=dev)
-                if _use_tc(D, C):
-                    img = torch.empty(lib.mrb_gemm_tc_image_bytes(D, C), dtype=torch.uint8, device=dev)
-                    _lib.call("mrb_gemm_tc_pack", w.data_ptr() + 4 * c0, None, ctot, 1, 0, 0, D, C, _lib.ptr(img))
-                    tc_gemm(gt_ptr, D, R, D, img, C, _lib.ptr(g_rows), C)
-                else:
-                    _gemm(False, False, R, C, D, gt_ptr, D, w.data_ptr() + 4 * c0, ctot, 0.0, _lib.ptr(g_rows), C)
-                g = torch.empty(shape, dtype=torch.float32, device=dev)
-                _lib.call("mrb_rows_to_feature_map", _lib.ptr(g_rows), C, n_img, C, R // n_img, _lib.ptr(g))
-                gmaps.append(g if dtypes[i] == torch.float32 else g.to(dtypes[i]))
-            else:
-                gmaps.append(None)
-            r0 += R
-            c0 += C
-        if gwt is not None:
-            gw = gwt.t().contiguous()       # nn.Linear stores out x in
+        gw, gmaps = _backproject_texels(gT, w, rows_cl, shapes, rows_per_map, dtypes, n_img, ctx.needs_input_grad[3],
+                                        ctx.needs_input_grad[4:])
         return (None, None, None, gw) + tuple(gmaps)
 
 
+class _VertAlignLinearBilinear(torch.autograd.Function):
+    """linear(bilinear VertexAlign(maps)) = sum over maps of bilinear(T_m)(v): the same per-texel projections T as
+    ``_VertAlignLinear``, then one bilinear sample of T_m per map, accumulated (csrc/vert_align_bilinear.cu).  The backward
+    kernel gives gT and the position gradient; the weight and map gradients come from gT as in ``_VertAlignLinear``."""
+
+    @staticmethod
+    def forward(ctx, pos, vert_mesh, mesh_info, weight, *fmaps):
+        _require_cuda(pos, "VertexAlign+linear")
+        dev = pos.device
+        pos_c = _f32c(pos.detach())
+        w, maps, n_img = _linear_maps(weight, fmaps)
+        D = w.shape[0]
+        T, rows_cl, rows_per_map = _project_texels(maps, w, n_img)
+        SV = pos_c.shape[0]
+        out = torch.empty(SV, D, dtype=torch.float32, device=dev)
+        r0 = 0
+        for i, (m, R) in enumerate(zip(maps, rows_per_map)):
+            _lib.call("mrb_vert_align_bilinear_fwd", T.data_ptr() + 4 * r0 * D, D, D, int(m.shape[2]), n_img, _lib.ptr(pos_c),
+                      _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, int(i > 0), _lib.ptr(out), D)
+            r0 += R
+        ctx.save_for_backward(pos_c, vert_mesh, mesh_info, w, T, *rows_cl)
+        ctx.meta = (n_img, [tuple(m.shape) for m in maps], [f.dtype for f in fmaps], rows_per_map, pos.dtype)
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        pos_c, vert_mesh, mesh_info, w, T = ctx.saved_tensors[:5]
+        rows_cl = ctx.saved_tensors[5:]
+        n_img, shapes, dtypes, rows_per_map, pos_dtype = ctx.meta
+        dev = gout.device
+        D = w.shape[0]
+        gout = _rows(gout)
+        SV = gout.shape[0]
+        want_T = ctx.needs_input_grad[3] or any(ctx.needs_input_grad[4:])
+        gT = torch.zeros(sum(rows_per_map), D, dtype=torch.float32, device=dev) if want_T else None
+        gpos = torch.zeros(SV, 3, dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
+        if gT is not None or gpos is not None:
+            r0 = 0
+            for shape, R in zip(shapes, rows_per_map):
+                _lib.call("mrb_vert_align_bilinear_bwd", gout.data_ptr(), gout.stride(0), T.data_ptr() + 4 * r0 * D, D, D,
+                          shape[2], n_img, _lib.ptr(pos_c), _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV,
+                          None if gT is None else gT.data_ptr() + 4 * r0 * D, D, _lib.ptr(gpos), 1)
+                r0 += R
+        gw, gmaps = None, [None] * len(shapes)
+        if gT is not None:
+            gw, gmaps = _backproject_texels(gT, w, rows_cl, shapes, rows_per_map, dtypes, n_img, ctx.needs_input_grad[3],
+                                            ctx.needs_input_grad[4:])
+        if gpos is not None and pos_dtype != torch.float32:
+            gpos = gpos.to(pos_dtype)
+        return (gpos, None, None, gw) + tuple(gmaps)
+
+
 def vert_align_linear(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
-                      image_sizes, mesh_index: Sequence[int], weight: Tensor, topo: Optional[MeshTopology] = None) -> Tensor:
+                      image_sizes, mesh_index: Sequence[int], weight: Tensor, topo: Optional[MeshTopology] = None,
+                      bilinear: bool = False) -> Tensor:
     """``F.linear(VertexAlign()(img_features, ...), weight)`` (weight: out x sum(C_m), no bias) without forming the
-    SV x sum(C_m) matrix -- see ``_VertAlignLinear``."""
+    SV x sum(C_m) matrix -- see ``_VertAlignLinear``.  ``bilinear=True``: the same with bilinear VertexAlign
+    (``vert_align_bilinear``), differentiable in ``vertex_positions`` too (``_VertAlignLinearBilinear``)."""
+    if bilinear:
+        vert_mesh, info = _bilinear_tables(img_features, vertex_positions, vertices_per_mesh, mesh_index, image_sizes)
+        return _VertAlignLinearBilinear.apply(vertex_positions, vert_mesh, info, weight, *img_features)
     dev = vertex_positions.device
     _require_cuda(vertex_positions, "VertexAlign")
     if sum(int(m) for m in mesh_index) != len(vertices_per_mesh):

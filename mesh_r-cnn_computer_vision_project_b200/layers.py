@@ -74,13 +74,26 @@ class VoxelBranch(nn.Sequential):
         return x
 
 
+ALIGN_MODES = ("reference", "bilinear")
+
+
 class VertexAlign(nn.Module):
     """Projects mesh vertices into the image plane and pools feature-map texels.
 
     Mirrors reference ``VertexAlign.forward(img_features, vertex_positions, vertices_per_mesh, image_sizes,
     mesh_index)`` (meshRCNN/layers.py:521-546) including its actual arithmetic (:557-611): fixed intrinsics
     (248, 111.5), clamp to the image, nearest-floor texel with the H/W axes swapped, 0/1 mask, no gradient to the
-    positions.  Output: SV x sum(C_m)."""
+    positions.  Output: SV x sum(C_m).
+
+    ``mode="bilinear"`` (opt-in, a plain attribute that may also be set on a loaded model): the same projection, then a
+    bilinear sample of each map (``functional.vert_align_bilinear``), differentiable in the maps and in the vertex
+    positions.  No parameters or buffers either way, so state dicts do not depend on the mode."""
+
+    def __init__(self, mode: str = "reference"):
+        super().__init__()
+        if mode not in ALIGN_MODES:
+            raise ValueError("VertexAlign: mode must be one of %s, got %r" % (ALIGN_MODES, mode))
+        self.mode = mode
 
     def forward(self, img_features: List[Tensor], vertex_positions: Tensor, vertices_per_mesh: List[int],
                 image_sizes: List[Tuple[int, int]], mesh_index: List[int]) -> Tensor:
@@ -88,7 +101,16 @@ class VertexAlign(nn.Module):
             assert len(vertices_per_mesh) == len(image_sizes)
             assert list(mesh_index) == [1 for _ in image_sizes]
         assert len(mesh_index) == len(image_sizes)              # layers.py:532
+        if _bilinear(self):
+            return F_.vert_align_bilinear(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index)
         return F_.vert_align(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index)
+
+
+def _bilinear(align: VertexAlign) -> bool:
+    mode = getattr(align, "mode", "reference")
+    if mode not in ALIGN_MODES:
+        raise ValueError("VertexAlign: mode must be one of %s, got %r" % (ALIGN_MODES, mode))
+    return mode == "bilinear"
 
 
 # Stage inputs are column concatenations [features | position | aligned features] (reference layers.py:160-165,241-252,
@@ -176,7 +198,8 @@ def _align_and_project(align: "VertexAlign", linear: nn.Linear, img_feature_maps
         assert len(vertice_index) == len(image_sizes)
         assert list(mesh_index) == [1 for _ in image_sizes]
     assert len(mesh_index) == len(image_sizes)
-    return F_.vert_align_linear(img_feature_maps, vertex_positions, vertice_index, image_sizes, mesh_index, linear.weight)
+    return F_.vert_align_linear(img_feature_maps, vertex_positions, vertice_index, image_sizes, mesh_index, linear.weight,
+                                bilinear=_bilinear(align))
 
 
 def _stage_input(vertex_positions, pooled, vertex_features, use_input_features):
@@ -206,9 +229,9 @@ class ResVertixRefineShapenet(nn.Module):
     NB the argument order of ``forward`` differs from the other two stage classes (:130-133)."""
 
     def __init__(self, use_input_features: bool = True, num_features: int = 128, alignment_size: int = 3840,
-                 ndims: int = 3):
+                 ndims: int = 3, align_mode: str = "reference"):
         super().__init__()
-        self.vertAlign = VertexAlign()
+        self.vertAlign = VertexAlign(align_mode)
         self.linear = _BiasFreeLinear(alignment_size, num_features)
         in_channels = num_features + ndims + (num_features if use_input_features else 0)
         self.resGraphConv0 = ResGraphConv(in_channels, num_features)
@@ -236,9 +259,9 @@ class VertixRefineShapeNet(nn.Module):
     """Plain ShapeNet refinement stage -- reference meshRCNN/layers.py:181-259."""
 
     def __init__(self, use_input_features: bool = True, num_features: int = 128, alignment_size: int = 3840,
-                 ndims: int = 3):
+                 ndims: int = 3, align_mode: str = "reference"):
         super().__init__()
-        self.vertAlign = VertexAlign()
+        self.vertAlign = VertexAlign(align_mode)
         self.linear0 = _BiasFreeLinear(alignment_size, num_features)
         in_channels = num_features + ndims + (num_features if use_input_features else 0)
         self.graphConv0 = GraphConv(in_channels, num_features)
@@ -268,9 +291,9 @@ class VertixRefinePix3D(nn.Module):
     """Pix3D refinement stage (single RoI feature map, no bottleneck) -- reference meshRCNN/layers.py:262-339."""
 
     def __init__(self, use_input_features: bool = True, num_features: int = 128, alignment_size: int = 256,
-                 ndims: int = 3):
+                 ndims: int = 3, align_mode: str = "reference"):
         super().__init__()
-        self.vertAlign = VertexAlign()
+        self.vertAlign = VertexAlign(align_mode)
         in_channels = alignment_size + ndims + (num_features if use_input_features else 0)
         self.graphConv0 = GraphConv(in_channels, num_features)
         self.use_input_features = use_input_features
@@ -283,7 +306,7 @@ class VertixRefinePix3D(nn.Module):
                 vertex_positions: Tensor, image_sizes: List, mesh_index: List[int] = None,
                 vertex_features: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
         mesh_index = _default_mesh_index(mesh_index, image_sizes)
-        if FUSE_STAGE_INPUTS and self.graphConv0.w0.shape[1] % 4 == 0:
+        if FUSE_STAGE_INPUTS and self.graphConv0.w0.shape[1] % 4 == 0 and not _bilinear(self.vertAlign):
             # VertexAlign stays factored: graphConv0 projects the texels and gathers rows (functional.TexelTerm)
             if self.vertAlign.training:                             # the checks of VertexAlign.forward (layers.py:528-532)
                 assert len(vertice_index) == len(image_sizes)
@@ -293,6 +316,7 @@ class VertixRefinePix3D(nn.Module):
             aligned = F_.TexelTerm(back_bone_features, vertex_positions, vertice_index, image_sizes, mesh_index,
                                    topo=topology.lookup(vertex_adjacency, vertex_positions.shape[0]))
         else:
+            # literal mode, and bilinear mode: the SV x C aligned features are materialised and enter as a dense part
             aligned = self.vertAlign([back_bone_features], vertex_positions, vertice_index, image_sizes, mesh_index)
         x = _stage_input(vertex_positions, aligned, vertex_features, self.use_input_features)
         x = self.graphConv0(x, vertex_adjacency)

@@ -40,10 +40,11 @@ class RefinementHead(nn.Module):
     ``refineStages.{i}.*`` as in shapenet_model.py:27-41 / pix3d_model.py:32-44).
 
     ``model``: "pix3d" (VertixRefinePix3D, 256-channel RoI map), "shapenet" (VertixRefineShapeNet) or
-    "shapenet_residual" (ResVertixRefineShapenet)."""
+    "shapenet_residual" (ResVertixRefineShapenet).  ``align_mode``: "reference" (the reference's VertexAlign arithmetic) or
+    "bilinear" (bilinear sampling with gradients to the vertex positions, ``layers.VertexAlign``)."""
 
     def __init__(self, model: str = "pix3d", cubify_threshold: float = 0.2, alignment_channels: Optional[int] = None,
-                 vertex_feature_dim: int = 128, num_refinement_stages: int = 3):
+                 vertex_feature_dim: int = 128, num_refinement_stages: int = 3, align_mode: str = "reference"):
         super().__init__()
         cls = {"pix3d": VertixRefinePix3D, "shapenet": VertixRefineShapeNet,
                "shapenet_residual": ResVertixRefineShapenet}[model]
@@ -51,10 +52,11 @@ class RefinementHead(nn.Module):
             alignment_channels = 256 if model == "pix3d" else 3840
         self.model = model
         self.cubify = Cubify(cubify_threshold)
-        stages = [cls(alignment_size=alignment_channels, use_input_features=False, num_features=vertex_feature_dim)]
+        stages = [cls(alignment_size=alignment_channels, use_input_features=False, num_features=vertex_feature_dim,
+                      align_mode=align_mode)]
         for _ in range(num_refinement_stages - 1):
             stages.append(cls(alignment_size=alignment_channels, use_input_features=True,
-                              num_features=vertex_feature_dim))
+                              num_features=vertex_feature_dim, align_mode=align_mode))
         self.refineStages = nn.ModuleList(stages)
         self.overlap_losses = True          # training: per-stage losses on a second CUDA stream (see forward)
         self._loss_stream = None
