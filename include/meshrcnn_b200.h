@@ -57,6 +57,19 @@ int mrb_cubify_count(const float* probs, int B, int Z, int Y, int X, float thres
 int mrb_cubify_emit(int B, int Z, int Y, int X, void* workspace, const long long* meta, long long SV, long long SF,
                     long long E, float* verts, long long* faces, long long* adj, int32_t* rowptr, int32_t* col32,
                     int32_t* vert_mesh, void* vert_aux, void* stream);
+/* The same two phases with a choice of quad placement; mrb_cubify_count / mrb_cubify_emit are these with topology 0.
+ *   topology 0 (reference): the reference's corner table, bit-exact -- dirs 2/3 place the quad on the side away from the
+ *     empty neighbour and c0..c3 are in lattice order, so the two triangles overlap with opposite winding.
+ *   topology 1 (watertight): each quad on the side of the empty neighbour, corners cyclic from its lowest lattice corner,
+ *     both triangles wound outward ((c1-c0) x (c2-c0) toward the empty neighbour): a closed surface per mesh whose fp64
+ *     signed volume equals its voxel count.  Same face flags, orders, coordinates, counts of faces and workspace size.
+ * Any other topology is rejected before a launch.  Precondition: the emit gets the topology the count got (the count's
+ * lattice masks in the workspace, hence its vertex and edge counts, depend on it). */
+int mrb_cubify_count_topo(const float* probs, int B, int Z, int Y, int X, float threshold, int from_logits, int topology,
+                          void* workspace, long long* meta, void* stream);
+int mrb_cubify_emit_topo(int B, int Z, int Y, int X, void* workspace, const long long* meta, long long SV, long long SF,
+                         long long E, float* verts, long long* faces, long long* adj, int32_t* rowptr, int32_t* col32,
+                         int32_t* vert_mesh, void* vert_aux, int topology, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Voxel-head tail (SURVEY 8 f-1) -- replaces nn.Sigmoid at the end of VoxelBranch (meshRCNN/layers.py:487-506) + voxel_loss

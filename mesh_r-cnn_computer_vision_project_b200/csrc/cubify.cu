@@ -39,6 +39,28 @@ __constant__ uint32_t kLatMask[8][6] = {
     {0x0000000u, 0x0009000u, 0x0001008u, 0x0000000u, 0x0000000u, 0x0000090u},
     {0x0000000u, 0x0004c00u, 0x0000000u, 0x0004030u, 0x0000412u, 0x0000000u},
     {0x0000000u, 0x0001200u, 0x0000000u, 0x0001008u, 0x0000000u, 0x0000012u}};
+// The same rule for the watertight topology (opt-in): quad on the side of the empty neighbour, corners cyclic from the
+// quad's lowest lattice corner with outward winding -- corner_id<kWatertight> below, oracle/cubify_watertight.py.
+// The triangles (c0,c1,c2),(c0,c2,c3) have the same five edges, so only the corner positions change the mask.
+__constant__ uint32_t kLatMaskWT[8][6] = {
+    {0x0034000u, 0x0000000u, 0x0000000u, 0x0c04000u, 0x2410000u, 0x0000000u},
+    {0x0011000u, 0x0000000u, 0x0000000u, 0x0401000u, 0x0000000u, 0x2410000u},
+    {0x0004400u, 0x0000000u, 0x0c04000u, 0x0000000u, 0x0400400u, 0x0000000u},
+    {0x0001600u, 0x0000000u, 0x0401000u, 0x0000000u, 0x0000000u, 0x0400400u},
+    {0x0000000u, 0x0034000u, 0x0000000u, 0x0004010u, 0x0010010u, 0x0000000u},
+    {0x0000000u, 0x0011000u, 0x0000000u, 0x0001018u, 0x0000000u, 0x0010010u},
+    {0x0000000u, 0x0004400u, 0x0004010u, 0x0000000u, 0x0000412u, 0x0000000u},
+    {0x0000000u, 0x0001600u, 0x0001018u, 0x0000000u, 0x0000000u, 0x0000412u}};
+
+// Quad placement, a compile-time choice of the two kernels that depend on it (k_lattice_count, k_emit_faces); every other
+// kernel works from the face flags and lattice masks and is shared.
+enum Topology { kReference = 0, kWatertight = 1 };
+
+template <int TOPO>
+__device__ __forceinline__ uint32_t lat_mask(int s, int k) {
+    if constexpr (TOPO == kWatertight) return kLatMaskWT[s][k];
+    else return kLatMask[s][k];
+}
 
 struct Dims {
     int B, Z, Y, X;
@@ -149,6 +171,7 @@ __device__ __forceinline__ uint32_t lattice_mask(const uint8_t* __restrict__ ffb
 }
 
 // pass 1b: per-(mesh, lattice chunk) vertex and directed-edge counts; the masks are kept for the emit pass
+template <int TOPO>
 __global__ void __launch_bounds__(CH) k_lattice_count(Dims d, Workspace ws) {
     __shared__ int scratch[33];
     __shared__ uint32_t tab[8][64];
@@ -157,7 +180,7 @@ __global__ void __launch_bounds__(CH) k_lattice_count(Dims d, Workspace ws) {
         uint32_t m = 0;
 #pragma unroll
         for (int k = 0; k < 6; ++k)
-            if ((f >> k) & 1) m |= kLatMask[s8][k];
+            if ((f >> k) & 1) m |= lat_mask<TOPO>(s8, k);
         tab[s8][f] = m;
     }
     __syncthreads();
@@ -324,12 +347,17 @@ __global__ void __launch_bounds__(ADJ_BLOCK) k_emit_adj(Dims d, Workspace ws, in
 // instruction bound (1 080 warp instructions per 32 voxels): now the 8 corner ranks of a voxel are loaded once (not 4 per
 // quad with their own index arithmetic), the quad corners are compile-time picks among them, and the per-warp output offsets
 // of all six directions come from one shared-memory prefix pass instead of a serial sum per (thread, direction).
+template <int TOPO>
 __device__ __forceinline__ constexpr int corner_id(int k, int j) {
     // kCorner[k][j] as cz*4 + cy*2 + cx (same table as the __constant__ one above, usable in constant expressions)
     constexpr int T[6][4] = {{0, 1, 2, 3}, {4, 5, 6, 7}, {4, 5, 0, 1}, {2, 3, 6, 7}, {4, 0, 6, 2}, {1, 5, 3, 7}};
-    return T[k][j];
+    // watertight: d0 000 001 011 010, d1 100 110 111 101, d2 010 011 111 110, d3 000 100 101 001, d4 000 010 110 100,
+    // d5 001 101 111 011 (z,y,x offsets; cyclic, (c1-c0) x (c2-c0) toward the empty neighbour)
+    constexpr int W[6][4] = {{0, 1, 3, 2}, {4, 6, 7, 5}, {2, 3, 7, 6}, {0, 4, 5, 1}, {0, 2, 6, 4}, {1, 5, 7, 3}};
+    return TOPO == kWatertight ? W[k][j] : T[k][j];
 }
 
+template <int TOPO>
 __global__ void __launch_bounds__(CH) k_emit_faces(Dims d, Workspace ws, const long long* __restrict__ meta,
                                                    long long* __restrict__ faces) {
     constexpr int NW = CH / 32;
@@ -365,7 +393,8 @@ __global__ void __launch_bounds__(CH) k_emit_faces(Dims d, Workspace ws, const l
     for (int k = 0; k < 6; ++k) {
         if (!((f >> k) & 1u)) continue;
         const long long q = ws.segBase[b] + ws.faceOff[((size_t)b * 6 + k) * d.nchF + chunk] + wtot[k][warp_id()] + pre[k];
-        const long long c0 = r[corner_id(k, 0)], c1 = r[corner_id(k, 1)], c2 = r[corner_id(k, 2)], c3 = r[corner_id(k, 3)];
+        const long long c0 = r[corner_id<TOPO>(k, 0)], c1 = r[corner_id<TOPO>(k, 1)], c2 = r[corner_id<TOPO>(k, 2)],
+                        c3 = r[corner_id<TOPO>(k, 3)];
         longlong2* o = reinterpret_cast<longlong2*>(faces + q * 6);          // 48-byte quads: 16-byte aligned
         o[0] = make_longlong2(c0, c1);
         o[1] = make_longlong2(c2, c0);
@@ -385,8 +414,9 @@ extern "C" long long mrb_cubify_workspace_bytes(int B, int Z, int Y, int X) {
     return (long long)carve(d, nullptr, nullptr);
 }
 
-extern "C" int mrb_cubify_count(const float* probs, int B, int Z, int Y, int X, float threshold, int from_logits,
-                                void* workspace, long long* meta, void* stream_) {
+extern "C" int mrb_cubify_count_topo(const float* probs, int B, int Z, int Y, int X, float threshold, int from_logits,
+                                     int topology, void* workspace, long long* meta, void* stream_) {
+    MRB_REQUIRE(topology == kReference || topology == kWatertight, "cubify_count: bad topology %d", topology);
     MRB_REQUIRE(probs && workspace && meta, "cubify_count: null pointer");
     MRB_REQUIRE(B > 0 && Z > 0 && Y > 0 && X > 0, "cubify_count: bad grid %dx%dx%dx%d", B, Z, Y, X);
     MRB_REQUIRE((long long)B * (Z + 1) * (Y + 1) * (X + 1) < (1LL << 31), "cubify_count: lattice too large for int32");
@@ -397,15 +427,23 @@ extern "C" int mrb_cubify_count(const float* probs, int B, int Z, int Y, int X, 
     carve(d, workspace, &ws);
     if (from_logits) k_faceflags<true><<<dim3(d.nchF, B), CH, 0, stream>>>(probs, threshold, d, ws);
     else k_faceflags<false><<<dim3(d.nchF, B), CH, 0, stream>>>(probs, threshold, d, ws);
-    k_lattice_count<<<dim3(d.nchL, B), CH, 0, stream>>>(d, ws);
+    if (topology == kWatertight) k_lattice_count<kWatertight><<<dim3(d.nchL, B), CH, 0, stream>>>(d, ws);
+    else k_lattice_count<kReference><<<dim3(d.nchL, B), CH, 0, stream>>>(d, ws);
     k_scan_seg<<<dim3(B, 3), SEG_THREADS, 0, stream>>>(d, ws);
     k_scan_top<<<3, 1024, 0, stream>>>(d, ws, meta);
     return check_launch("cubify_count");
 }
 
-extern "C" int mrb_cubify_emit(int B, int Z, int Y, int X, void* workspace, const long long* meta, long long SV,
-                               long long SF, long long E, float* verts, long long* faces, long long* adj,
-                               int32_t* rowptr, int32_t* col32, int32_t* vert_mesh, void* vert_aux, void* stream_) {
+extern "C" int mrb_cubify_count(const float* probs, int B, int Z, int Y, int X, float threshold, int from_logits,
+                                void* workspace, long long* meta, void* stream_) {
+    return mrb_cubify_count_topo(probs, B, Z, Y, X, threshold, from_logits, kReference, workspace, meta, stream_);
+}
+
+extern "C" int mrb_cubify_emit_topo(int B, int Z, int Y, int X, void* workspace, const long long* meta, long long SV,
+                                    long long SF, long long E, float* verts, long long* faces, long long* adj,
+                                    int32_t* rowptr, int32_t* col32, int32_t* vert_mesh, void* vert_aux, int topology,
+                                    void* stream_) {
+    MRB_REQUIRE(topology == kReference || topology == kWatertight, "cubify_emit: bad topology %d", topology);
     MRB_REQUIRE(workspace && meta && verts && faces && adj && rowptr && col32 && vert_mesh && vert_aux,
                 "cubify_emit: null pointer");
     MRB_REQUIRE(SV > 0 && SF > 0 && E > 0, "cubify_emit: empty grid");
@@ -417,6 +455,14 @@ extern "C" int mrb_cubify_emit(int B, int Z, int Y, int X, void* workspace, cons
     int32_t* vlat = (int32_t*)vert_aux + SV;
     k_emit_verts<<<dim3(d.nchL, B), CH, 0, stream>>>(d, ws, verts, rowptr, vert_mesh, vmask, vlat);
     k_emit_adj<<<ceil_div(SV, ADJ_BLOCK), ADJ_BLOCK, 0, stream>>>(d, ws, (int)SV, rowptr, vmask, vlat, adj, adj + E, col32);
-    k_emit_faces<<<dim3(d.nchF, B), CH, 0, stream>>>(d, ws, meta, faces);
+    if (topology == kWatertight) k_emit_faces<kWatertight><<<dim3(d.nchF, B), CH, 0, stream>>>(d, ws, meta, faces);
+    else k_emit_faces<kReference><<<dim3(d.nchF, B), CH, 0, stream>>>(d, ws, meta, faces);
     return check_launch("cubify_emit");
+}
+
+extern "C" int mrb_cubify_emit(int B, int Z, int Y, int X, void* workspace, const long long* meta, long long SV,
+                               long long SF, long long E, float* verts, long long* faces, long long* adj,
+                               int32_t* rowptr, int32_t* col32, int32_t* vert_mesh, void* vert_aux, void* stream_) {
+    return mrb_cubify_emit_topo(B, Z, Y, X, workspace, meta, SV, SF, E, verts, faces, adj, rowptr, col32, vert_mesh,
+                                vert_aux, kReference, stream_);
 }

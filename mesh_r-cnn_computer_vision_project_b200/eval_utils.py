@@ -155,8 +155,9 @@ def compare_meshes(pred_verts: Tensor, pred_faces: Tensor, pred_v_index: Sequenc
     - ``Precision@tau`` / ``Recall@tau`` = 100 x share of predicted / GT samples with sqrt(d) < tau, ``F1@tau`` =
       2PR / (P + R + 1e-8) for every threshold (at most 8).
 
-    Cubify emits the two triangles of a quad with opposite winding, so the signed ``NormalConsistency`` of cubified meshes
-    is dominated by that flip; ``AbsNormalConsistency`` is the meaningful one for them.
+    Cubify's reference topology emits the two triangles of a quad with opposite winding, so the signed ``NormalConsistency``
+    of such meshes is dominated by that flip; ``AbsNormalConsistency`` is the meaningful one for them.  Meshes of
+    ``Cubify(topology="watertight")`` are wound outward throughout, and their signed ``NormalConsistency`` is meaningful.
 
     B is ``len(gt_f_index)``; shorter prediction lists (Cubify drops trailing empty meshes) are padded with empty meshes.  A
     predicted mesh without faces is invalid: NaN Chamfer / NC / AbsNC, 0 for P / R / F1.  Randomness: ``seed`` (predicted

@@ -7,6 +7,7 @@ caller's current stream through ``_lib.call``.
 import ctypes
 import os
 import threading
+import weakref
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -20,6 +21,14 @@ CUBIFY_CORNERS = (
     ((0, 0, 0), (0, 0, 1), (0, 1, 0), (0, 1, 1)), ((1, 0, 0), (1, 0, 1), (1, 1, 0), (1, 1, 1)),
     ((1, 0, 0), (1, 0, 1), (0, 0, 0), (0, 0, 1)), ((0, 1, 0), (0, 1, 1), (1, 1, 0), (1, 1, 1)),
     ((1, 0, 0), (0, 0, 0), (1, 1, 0), (0, 1, 0)), ((0, 0, 1), (1, 0, 1), (0, 1, 1), (1, 1, 1)))
+
+# Cubify quad placements, by the ``topology`` value of mrb_cubify_count_topo / mrb_cubify_emit_topo
+CUBIFY_TOPOLOGIES = ("reference", "watertight")
+
+
+def check_cubify_topology(topology: str) -> None:
+    if topology not in CUBIFY_TOPOLOGIES:
+        raise ValueError("Cubify: topology must be one of %s, got %r" % (CUBIFY_TOPOLOGIES, topology))
 
 
 def _require_cuda(t: Tensor, what: str) -> None:
@@ -52,9 +61,13 @@ def _pinned_i64(n: int, device) -> Tensor:
 
 
 @torch.no_grad()
-def cubify(t: Tensor, threshold: float, from_logits: bool = False):
+def cubify(t: Tensor, threshold: float, from_logits: bool = False, topology: str = "reference"):
     """See ``layers.Cubify``.  Returns (verts, v_index, faces, f_index, adj, topology).  ``from_logits``: ``t`` holds the
-    voxel head's logits and ``sigmoid(t) > threshold`` is tested inside the first kernel (SURVEY 8 f-1)."""
+    voxel head's logits and ``sigmoid(t) > threshold`` is tested inside the first kernel (SURVEY 8 f-1).  ``topology``:
+    "reference" (the reference's quads, bit-exact) or "watertight" (closed, outward-wound cube surfaces, DESIGN.md §2
+    item 8); the returned ``topology`` is the adjacency's CSR form, whichever the quad placement."""
+    check_cubify_topology(topology)
+    watertight = topology == "watertight"
     _require_cuda(t, "Cubify")
     if t.dim() != 4:
         raise RuntimeError("Cubify expects B x Z x Y x X, got %s" % (tuple(t.shape),))
@@ -68,8 +81,12 @@ def cubify(t: Tensor, threshold: float, from_logits: bool = False):
             raise RuntimeError("Cubify: bad grid shape %s" % (tuple(t.shape),))
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         meta = torch.empty(4 + 4 * B, dtype=torch.int64, device=dev)
-        _lib.call("mrb_cubify_count", _lib.ptr(probs), B, Z, Y, X, float(threshold), int(bool(from_logits)), _lib.ptr(ws),
-                  _lib.ptr(meta))
+        if watertight:
+            _lib.call("mrb_cubify_count_topo", _lib.ptr(probs), B, Z, Y, X, float(threshold), int(bool(from_logits)), 1,
+                      _lib.ptr(ws), _lib.ptr(meta))
+        else:
+            _lib.call("mrb_cubify_count", _lib.ptr(probs), B, Z, Y, X, float(threshold), int(bool(from_logits)),
+                      _lib.ptr(ws), _lib.ptr(meta))
         # The one unavoidable sync: the API returns Python lists.  The counters are copied into pinned memory asynchronously;
         # work that does not depend on the mesh (the texel projections of the pass, functional.PackPlan) is launched behind
         # the copy, so the device has something to do while this thread waits, allocates and issues the emit kernels.
@@ -92,9 +109,12 @@ def cubify(t: Tensor, threshold: float, from_logits: bool = False):
         col32 = torch.empty(E, dtype=torch.int32, device=dev)
         vert_mesh = torch.empty(SV, dtype=torch.int32, device=dev)
         aux = torch.empty(2 * SV, dtype=torch.int32, device=dev)
-        _lib.call("mrb_cubify_emit", B, Z, Y, X, _lib.ptr(ws), _lib.ptr(meta), SV, SF, E, _lib.ptr(verts),
-                  _lib.ptr(faces), _lib.ptr(adj), _lib.ptr(rowptr), _lib.ptr(col32), _lib.ptr(vert_mesh),
-                  _lib.ptr(aux))
+        out = (_lib.ptr(verts), _lib.ptr(faces), _lib.ptr(adj), _lib.ptr(rowptr), _lib.ptr(col32), _lib.ptr(vert_mesh),
+               _lib.ptr(aux))
+        if watertight:
+            _lib.call("mrb_cubify_emit_topo", B, Z, Y, X, _lib.ptr(ws), _lib.ptr(meta), SV, SF, E, *out, 1)
+        else:
+            _lib.call("mrb_cubify_emit", B, Z, Y, X, _lib.ptr(ws), _lib.ptr(meta), SV, SF, E, *out)
     topo = MeshTopology(SV, E, rowptr, col32, symmetric=True, vert_mesh=vert_mesh)
     register(adj, topo)
     return verts, v_counts[:last], faces, f_counts[:last], adj, topo
@@ -442,16 +462,17 @@ _ROWS_CACHE = {}
 def feature_rows(fmap: Tensor) -> Tensor:
     """Channels-last fp32 rows (n_img * H * W x C) of an NCHW fp32 / bf16 feature map: the A operand of the per-texel
     projections.  The three stages of a forward pass read the same map, so the last conversion is cached by tensor identity
-    and version."""
+    and version.  Identity is a weak reference, not the address: a new map allocated where a freed one lived must not get
+    the freed map's rows."""
     key = (fmap.data_ptr(), fmap._version, tuple(fmap.shape), fmap.dtype, fmap.device.index)
     hit = _ROWS_CACHE.get("last")
-    if hit is not None and hit[0] == key:
+    if hit is not None and hit[0] == key and hit[2]() is fmap:
         return hit[1]
     m = _map_tensor(fmap.detach())
     n_img, C, H, W = m.shape
     rows = torch.empty(n_img * H * W, C, dtype=torch.float32, device=m.device)
     _lib.call("mrb_feature_map_to_rows", _lib.ptr(m), int(m.dtype == torch.bfloat16), n_img, C, H * W, _lib.ptr(rows))
-    _ROWS_CACHE["last"] = (key, rows)
+    _ROWS_CACHE["last"] = (key, rows, weakref.ref(fmap))
     return rows
 
 

@@ -26,11 +26,18 @@ class Cubify(nn.Module):
     mesh, like ``bincount``); ``faces`` SF x 3 int64 with per-mesh local vertex ids; ``adj_index`` 2 x E int64 with
     global ids sorted by (row, col).  Vertex / face / edge order equals the reference's (bit-exact).
     Raises ``ValueError("empty grid")`` when no voxel of the whole batch is occupied (layers.py:434-435).
+
+    ``topology="watertight"`` (opt-in, a plain attribute that may also be set on a loaded model): every quad on the side of
+    its empty neighbour, split along a diagonal into two outward-wound triangles, so each mesh is a closed surface (signed
+    volume = voxel count) and the graph has no spurious diagonals or interior vertices.  Same orders, coordinates and
+    face counts; fewer vertices and edges.  The buffers (and state-dict keys) do not depend on the topology.
     """
 
-    def __init__(self, threshold: float = 0.5):
+    def __init__(self, threshold: float = 0.5, topology: str = "reference"):
         super().__init__()
+        F_.check_cubify_topology(topology)
         self.threshold = threshold
+        self.topology = topology
         # state-dict compatibility with the reference ("cubify.kernel", "cubify.deltas", layers.py:365,401);
         # the CUDA path does not read them (the same tables live in csrc/cubify.cu as constants).
         nbr = [(-1, 0, 0), (1, 0, 0), (0, 1, 0), (0, -1, 0), (0, 0, -1), (0, 0, 1)]
@@ -50,7 +57,8 @@ class Cubify(nn.Module):
     def forward(self, t: Tensor, from_logits: bool = False):
         """``from_logits=True`` (extension, SURVEY 8 f-1): ``t`` holds the voxel head's logits; ``sigmoid(t) > threshold`` is
         evaluated inside the first kernel, so the probability grid is never written."""
-        verts, v_index, faces, f_index, adj, _ = F_.cubify(t, float(self.threshold), from_logits)
+        verts, v_index, faces, f_index, adj, _ = F_.cubify(t, float(self.threshold), from_logits,
+                                                           getattr(self, "topology", "reference"))
         return verts, v_index, faces, f_index, adj
 
 

@@ -41,17 +41,19 @@ class RefinementHead(nn.Module):
 
     ``model``: "pix3d" (VertixRefinePix3D, 256-channel RoI map), "shapenet" (VertixRefineShapeNet) or
     "shapenet_residual" (ResVertixRefineShapenet).  ``align_mode``: "reference" (the reference's VertexAlign arithmetic) or
-    "bilinear" (bilinear sampling with gradients to the vertex positions, ``layers.VertexAlign``)."""
+    "bilinear" (bilinear sampling with gradients to the vertex positions, ``layers.VertexAlign``).  ``cubify_topology``:
+    "reference" (the reference's Cubify, bit-exact) or "watertight" (closed cube meshes, ``layers.Cubify``)."""
 
     def __init__(self, model: str = "pix3d", cubify_threshold: float = 0.2, alignment_channels: Optional[int] = None,
-                 vertex_feature_dim: int = 128, num_refinement_stages: int = 3, align_mode: str = "reference"):
+                 vertex_feature_dim: int = 128, num_refinement_stages: int = 3, align_mode: str = "reference",
+                 cubify_topology: str = "reference"):
         super().__init__()
         cls = {"pix3d": VertixRefinePix3D, "shapenet": VertixRefineShapeNet,
                "shapenet_residual": ResVertixRefineShapenet}[model]
         if alignment_channels is None:
             alignment_channels = 256 if model == "pix3d" else 3840
         self.model = model
-        self.cubify = Cubify(cubify_threshold)
+        self.cubify = Cubify(cubify_threshold, topology=cubify_topology)
         stages = [cls(alignment_size=alignment_channels, use_input_features=False, num_features=vertex_feature_dim,
                       align_mode=align_mode)]
         for _ in range(num_refinement_stages - 1):
