@@ -187,36 +187,23 @@ int mrb_head_bwd(const float* g, const float* delta, const float* W, int ld_w, i
 
 /* ------------------------------------------------------------------------------------------------------------
  * VertexAlign -- replaces VertexAlign.forward / single_projection / project, reference meshRCNN/layers.py:521-613,
- * with the reference's exact (non-bilinear) semantics: out[v,c] = fmap[img,c,x1,y1] * [x2>x1 && y2>y1].
- *   fmap       n_img x C x Hm x Wm fp32 (NCHW, Hm == Wm)
- *   pos        SV x 3;  vert_mesh[v] = mesh of vertex v;  mesh_info[mesh] = {image index, image H, image W}
- *   out        SV x ld_out (this map's channels are written at out[v*ld_out + 0..C-1]; pass a column-offset pointer)
- *   workspace  n_img*C*Hm*Wm floats (channels-last copy of the map for the TMA bulk-copy gather); NULL selects the
- *              register path
- * Backward: gfmap[img,c,x1,y1] += gout[v,c] (atomic fp32); vertex positions receive no gradient (as in the
- * reference, where the integer cast at layers.py:592 cuts the graph).
- */
-int mrb_vert_align_fwd(const float* fmap, int n_img, int C, int Hm, int Wm, const float* pos, const int32_t* vert_mesh,
-                       const int32_t* mesh_info, int SV, float* out, int ld_out, float* workspace, void* stream);
-int mrb_vert_align_bwd(const float* gout, int ld_g, int n_img, int C, int Hm, int Wm, const float* pos,
-                       const int32_t* vert_mesh, const int32_t* mesh_info, int SV, float* gfmap, void* stream);
-
-/* bf16 feature-map mode (north star: "bf16 features rtol 2e-2"): fmap is n_img x C x Hm x Wm bf16 (NCHW); the output
- * stays fp32.  workspace: n_img*C*Hm*Wm bf16 elements (channels-last copy; NULL or C % 8 != 0 selects the
- * lane-per-channel path).  The backward is mrb_vert_align_bwd into an fp32 gradient map (the caller casts). */
-int mrb_vert_align_fwd_bf16(const void* fmap, int n_img, int C, int Hm, int Wm, const float* pos, const int32_t* vert_mesh,
-                            const int32_t* mesh_info, int SV, float* out, int ld_out, void* workspace, void* stream);
-
-/* VertexAlign fused with the bias-free linear layer that follows it in the ShapeNet stages (reference
- * meshRCNN/layers.py:115,151-155 and :192,230):  linear(align(f))[v] = sum_m mask_{v,m} * T_m[img(v)*HW_m + texel_m(v)]
- * with T_m = rows(f_m) @ W_m^T the per-texel projections (computed once per step with mrb_gemm_tc).
+ * with the reference's exact (non-bilinear) semantics: out[v,c] = fmap[img,c,x1,y1] * [x2>x1 && y2>y1], as a gather of
+ * channels-last texel rows.
+ *   pos        SV x 3;  vert_mesh[v] = mesh of vertex v;  mesh_info[mesh] = {image index, image H, image W}.  Every image
+ *              index must be < n_img: the caller validates it, the kernels do not clamp it.
  *   mrb_feature_map_to_rows   NCHW map (dtype 0 = fp32, 1 = bf16) -> channels-last fp32 rows (n_img*HW x C)
  *   mrb_rows_to_feature_map   channels-last fp32 rows (pitch ld_rows) -> NCHW fp32 (gradient of a map)
- *   mrb_vert_align_proj_fwd   T: packed texel projections, map m occupying rows [n_img * sum_{m'<m} HW_m', ...) in
- *                             (image, x1, y1) order, D columns; map_size_host: n_maps (<= 8) map sizes Hm == Wm, a HOST
- *                             array (read during the call);  out[v, 0:D] = sum_m mask * T[row_m(v)]
+ *   mrb_vert_align_proj_fwd   T: packed texel rows, map m occupying rows [n_img * sum_{m'<m} HW_m', ...) in (image, x1, y1)
+ *                             order, D columns; map_size_host: n_maps (<= 8) map sizes Hm == Wm, a HOST array (read during
+ *                             the call);  out[v, 0:D] = sum_m mask * T[row_m(v)], out rows of pitch ld_out (pass a
+ *                             column-offset pointer to fill a column block)
  *   mrb_vert_align_proj_bwd   gT (same shape as T, overwritten): gT[row_m(v)] += mask * gout[v]  (fp32 reductions)
- * D % 4 == 0; T, gT, out rows 16-byte aligned.  Vertex positions receive no gradient (layers.py:592). */
+ * The VertexAlign module calls the gather with one map, T = the map's rows and D = C.  Fused with the bias-free linear layer
+ * that follows it in the ShapeNet stages (reference meshRCNN/layers.py:115,151-155 and :192,230), T_m = rows(f_m) @ W_m^T
+ * are the per-texel projections (computed once per step with mrb_gemm_tc):  linear(align(f))[v] = sum_m mask_{v,m} *
+ * T_m[img(v)*HW_m + texel_m(v)].  float4 path when D % 4 == 0 and T / gT / out rows are 16-byte aligned, scalar otherwise;
+ * the forward of one such map (D <= 4096) moves whole rows with TMA bulk copies.
+ * Vertex positions receive no gradient (as in the reference, where the integer cast at layers.py:592 cuts the graph). */
 int mrb_feature_map_to_rows(const void* fmap, int dtype, int n_img, int C, int HW, float* rows, void* stream);
 int mrb_rows_to_feature_map(const float* rows, int ld_rows, int n_img, int C, int HW, float* gfmap, void* stream);
 int mrb_vert_align_proj_fwd(const float* T, int D, int n_maps, const int* map_size_host, int n_img, const float* pos,
@@ -227,7 +214,7 @@ int mrb_vert_align_proj_bwd(const float* gout, int ld_g, int D, int n_maps, cons
 
 /* Bilinear VertexAlign (opt-in mode; csrc/vert_align_bilinear.cu), differentiable in the vertex positions.  One square S x S
  * map given as channels-last fp32 rows: texel (i, j) of image img is rows[((img * S + i) * S + j) * ld_rows + 0 .. D-1] (the
- * output of mrb_feature_map_to_rows, or per-texel projections T of it).  Projection as mrb_vert_align_fwd up to and including
+ * output of mrb_feature_map_to_rows, or per-texel projections T of it).  Projection as mrb_vert_align_proj_fwd up to and including
  * the clamps to the image (x = w / sx indexes the H axis, y = h / sy the W axis), then x, y clamped to [0, S-1] and
  *   out[v] = (1-fx)(1-fy) f[x0,y0] + (1-fx) fy f[x0,y0+1] + fx (1-fy) f[x0+1,y0] + fx fy f[x0+1,y0+1]
  * with x0 = clamp(floor(x), 0, S-2), fx = x - x0 (y0, fy alike); S == 1 gives f[0,0].  This is grid_sample(align_corners=True,

@@ -1,4 +1,4 @@
-// Camera projection shared by the VertexAlign kernels (vert_align.cu, align_proj.cu).
+// Camera projection shared by the reference-mode VertexAlign kernels (align_proj.cu, graphconv2.cu).
 #pragma once
 #include "common.cuh"
 

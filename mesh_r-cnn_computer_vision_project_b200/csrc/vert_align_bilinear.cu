@@ -1,5 +1,5 @@
 // Bilinear VertexAlign over channels-last fp32 rows, with gradients to the rows and to the vertex positions (opt-in mode;
-// the reference-mode kernels in vert_align.cu / align_proj.cu / graphconv2.cu are separate and unchanged).
+// the reference-mode kernels in align_proj.cu / graphconv2.cu are separate and unchanged).
 //
 // For vertex v of mesh m, image img = mesh_info[m] and one square S x S map whose texel (i, j) of image img is the D-wide
 // row rows[(img * S + i) * S + j]:

@@ -115,7 +115,7 @@ def cubify(t: Tensor, threshold: float, from_logits: bool = False, topology: str
             _lib.call("mrb_cubify_emit_topo", B, Z, Y, X, _lib.ptr(ws), _lib.ptr(meta), SV, SF, E, *out, 1)
         else:
             _lib.call("mrb_cubify_emit", B, Z, Y, X, _lib.ptr(ws), _lib.ptr(meta), SV, SF, E, *out)
-    topo = MeshTopology(SV, E, rowptr, col32, symmetric=True, vert_mesh=vert_mesh)
+    topo = MeshTopology(SV, E, rowptr, col32, symmetric=True, vert_mesh=vert_mesh, v_index=v_counts[:last])
     register(adj, topo)
     return verts, v_counts[:last], faces, f_counts[:last], adj, topo
 
@@ -185,7 +185,9 @@ def offsets_table(counts: Sequence[int], device) -> Tensor:
 
 
 def vertex_mesh_ids(v_index: Sequence[int], num_vertices: int, device, topo: Optional[MeshTopology] = None) -> Tensor:
-    if topo is not None and topo.vert_mesh is not None and topo.num_vertices == num_vertices:
+    """int32 [num_vertices]: the mesh of every vertex.  Cubify's topology already holds them; they are reused only for the
+    very ``v_index`` Cubify returned, since another mesh list with the same vertex total would index other meshes."""
+    if topo is not None and topo.vert_mesh is not None and topo.v_index == list(v_index):
         return topo.vert_mesh
     off = offsets_table(v_index, device)
     ids = torch.empty(num_vertices, dtype=torch.int32, device=device)
@@ -483,22 +485,12 @@ class TexelTerm:
 
     def __init__(self, fmap: Tensor, vertex_positions: Tensor, vertices_per_mesh: Sequence[int], image_sizes,
                  mesh_index: Sequence[int], topo: Optional[MeshTopology] = None):
-        _require_cuda(fmap, "VertexAlign")
-        _require_cuda(vertex_positions, "VertexAlign")
-        if fmap.dim() != 4 or fmap.shape[2] != fmap.shape[3]:
-            raise RuntimeError("VertexAlign: feature maps must be N x C x H x W with H == W (the reference indexes H with the "
-                               "x coordinate)")
-        if sum(int(m) for m in mesh_index) != len(vertices_per_mesh):
-            raise RuntimeError("VertexAlign: sum(mesh_index) must equal the number of meshes")
-        if sum(vertices_per_mesh) != vertex_positions.shape[0]:
-            raise RuntimeError("VertexAlign: vertices_per_mesh does not sum to the number of vertex positions")
+        vert_mesh, info = align_tables([fmap], vertex_positions, vertices_per_mesh, image_sizes, mesh_index, topo)
         dev = vertex_positions.device
         SV = vertex_positions.shape[0]
         self.fmap = fmap
         self.n_img, self.C, self.size = int(fmap.shape[0]), int(fmap.shape[1]), int(fmap.shape[2])
         self.rows = feature_rows(fmap)
-        vert_mesh = vertex_mesh_ids(vertices_per_mesh, SV, dev, topo)
-        info = mesh_info_table(mesh_index, image_sizes, dev)
         self.texrow = torch.empty(SV, dtype=torch.int32, device=dev)
         _lib.call("mrb_vert_align_texrows", _lib.ptr(_f32c(vertex_positions.detach())), _lib.ptr(vert_mesh), _lib.ptr(info), SV,
                   self.size, _lib.ptr(self.texrow))
@@ -947,115 +939,70 @@ def _map_tensor(f: Tensor) -> Tensor:
     return _f32c(f)
 
 
-class _VertAlign(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, pos, vert_mesh, mesh_info, *fmaps):
-        _require_cuda(pos, "VertexAlign")
-        pos_c = _f32c(pos.detach())
-        maps = []
-        for f in fmaps:
-            _require_cuda(f, "VertexAlign")
-            if f.dim() != 4:
-                raise RuntimeError("VertexAlign: feature maps must be N x C x H x W")
-            maps.append(_map_tensor(f))
-        SV = pos_c.shape[0]
-        ctot = sum(m.shape[1] for m in maps)
-        out = torch.empty(SV, ctot, dtype=torch.float32, device=pos.device)
-        off = 0
-        for m in maps:
-            n_img, C, Hm, Wm = m.shape
-            ws = torch.empty_like(m)          # channels-last copy for the row gather
-            name = "mrb_vert_align_fwd_bf16" if m.dtype == torch.bfloat16 else "mrb_vert_align_fwd"
-            _lib.call(name, _lib.ptr(m), n_img, C, Hm, Wm, _lib.ptr(pos_c), _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV,
-                      _lib.ptr(out) + 4 * off, ctot, _lib.ptr(ws))
-            off += C
-        ctx.save_for_backward(pos_c, vert_mesh, mesh_info)
-        ctx.shapes = [tuple(m.shape) for m in maps]
-        ctx.dtypes = [f.dtype for f in fmaps]
-        return out
-
-    @staticmethod
-    def backward(ctx, gout):
-        pos_c, vert_mesh, mesh_info = ctx.saved_tensors
-        gout = _rows(gout)                       # usually a column slice of a stage-input gradient: read in place
-        SV, ctot = gout.shape
-        ldg = gout.stride(0)
-        grads = []
-        off = 0
-        for i, shape in enumerate(ctx.shapes):
-            n_img, C, Hm, Wm = shape
-            if ctx.needs_input_grad[3 + i]:
-                g = torch.zeros(shape, dtype=torch.float32, device=gout.device)
-                _lib.call("mrb_vert_align_bwd", gout.data_ptr() + 4 * off, ldg, n_img, C, Hm, Wm, _lib.ptr(pos_c),
-                          _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, _lib.ptr(g))
-                grads.append(g.to(ctx.dtypes[i]))
-            else:
-                grads.append(None)
-            off += C
-        return (None, None, None) + tuple(grads)   # no gradient to positions (reference layers.py:592)
-
-
-def vert_align(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
-               image_sizes, mesh_index: Sequence[int], topo: Optional[MeshTopology] = None) -> Tensor:
-    dev = vertex_positions.device
-    _require_cuda(vertex_positions, "VertexAlign")
-    if sum(int(m) for m in mesh_index) != len(vertices_per_mesh):
-        raise RuntimeError("VertexAlign: sum(mesh_index) must equal the number of meshes")
-    if sum(vertices_per_mesh) != vertex_positions.shape[0]:
-        raise RuntimeError("VertexAlign: vertices_per_mesh does not sum to the number of vertex positions")
-    vert_mesh = vertex_mesh_ids(vertices_per_mesh, vertex_positions.shape[0], dev, topo)
-    info = mesh_info_table(mesh_index, image_sizes, dev)
-    return _VertAlign.apply(vertex_positions, vert_mesh, info, *img_features)
-
-
-# ----------------------------------------------------------------------------------------------------------
-# bilinear VertexAlign (opt-in; csrc/vert_align_bilinear.cu): differentiable in the vertex positions
-# ----------------------------------------------------------------------------------------------------------
-def _square_maps(fmaps: Sequence[Tensor], what: str) -> List[Tensor]:
-    maps = []
-    for f in fmaps:
-        _require_cuda(f, what)
-        if f.dim() != 4 or f.shape[2] != f.shape[3]:
+def check_align_inputs(map_shapes, pos_shape, vertices_per_mesh: Sequence[int], image_sizes,
+                       mesh_index: Sequence[int]) -> None:
+    """The host-side checks of every VertexAlign entry point, on shapes and counts alone.  They keep every index the kernels
+    read in range: each vertex's mesh has a mesh_info row, and each image that holds a mesh exists in every map (the
+    reference raises IndexError there; the kernels do not clamp).  Raises RuntimeError."""
+    if len(pos_shape) != 2 or pos_shape[1] != 3:
+        raise RuntimeError("VertexAlign: vertex positions must be SV x 3")
+    for shape in map_shapes:
+        if len(shape) != 4 or shape[2] != shape[3]:
             raise RuntimeError("VertexAlign: feature maps must be N x C x H x W with H == W (the reference indexes H with the "
                                "x coordinate)")
-        maps.append(_map_tensor(f))
-    return maps
-
-
-def _bilinear_tables(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
-                     mesh_index: Sequence[int], image_sizes):
-    """(vert_mesh, mesh_info) of the bilinear kernels after the host-side checks that keep every index they read in range:
-    each vertex's mesh has a mesh_info row, and each image that holds a mesh exists in every map.  vert_mesh is built from
-    ``vertices_per_mesh`` itself (not taken from a registered topology), so it cannot name a mesh the table lacks."""
-    _require_cuda(vertex_positions, "VertexAlign")
-    if vertex_positions.dim() != 2 or vertex_positions.shape[1] != 3:
-        raise RuntimeError("VertexAlign: vertex positions must be SV x 3")
     if len(mesh_index) != len(image_sizes):
         raise RuntimeError("VertexAlign: mesh_index and image_sizes differ in length")
-    if any(int(m) < 0 for m in mesh_index) or any(int(c) < 0 for c in vertices_per_mesh):
+    if min(mesh_index, default=0) < 0 or min(vertices_per_mesh, default=0) < 0:
         raise RuntimeError("VertexAlign: negative mesh or vertex count")
-    if sum(int(m) for m in mesh_index) != len(vertices_per_mesh):
+    if sum(mesh_index) != len(vertices_per_mesh):
         raise RuntimeError("VertexAlign: sum(mesh_index) must equal the number of meshes")
-    if sum(int(c) for c in vertices_per_mesh) != vertex_positions.shape[0]:
+    if sum(vertices_per_mesh) != pos_shape[0]:
         raise RuntimeError("VertexAlign: vertices_per_mesh does not sum to the number of vertex positions")
-    used = [i for i, m in enumerate(mesh_index) if int(m) > 0]
+    last = len(mesh_index) - 1                          # the last image that holds a mesh
+    while last >= 0 and mesh_index[last] == 0:
+        last -= 1
+    for shape in map_shapes:
+        if last >= shape[0]:
+            raise RuntimeError("VertexAlign: image %d holds a mesh but the feature map has %d images" % (last, shape[0]))
+
+
+def align_tables(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int], image_sizes,
+                 mesh_index: Sequence[int], topo: Optional[MeshTopology] = None):
+    """(vert_mesh, mesh_info) of the VertexAlign kernels after every check: CUDA tensors on the current device, then
+    ``check_align_inputs``.  ``topo``: Cubify's topology, whose per-vertex mesh ids are reused for its own ``v_index``."""
+    _require_cuda(vertex_positions, "VertexAlign")
     for f in img_features:
-        if used and f.dim() == 4 and used[-1] >= f.shape[0]:
-            raise RuntimeError("VertexAlign: image %d holds a mesh but the feature map has %d images" % (used[-1], f.shape[0]))
+        _require_cuda(f, "VertexAlign")
+    check_align_inputs([tuple(f.shape) for f in img_features], tuple(vertex_positions.shape), vertices_per_mesh, image_sizes,
+                       mesh_index)
     dev = vertex_positions.device
     SV = vertex_positions.shape[0]
-    vert_mesh = vertex_mesh_ids(vertices_per_mesh, SV, dev) if SV else torch.empty(0, dtype=torch.int32, device=dev)
+    vert_mesh = vertex_mesh_ids(vertices_per_mesh, SV, dev, topo) if SV else torch.empty(0, dtype=torch.int32, device=dev)
     return vert_mesh, mesh_info_table(mesh_index, image_sizes, dev)
 
 
-class _VertAlignBilinear(torch.autograd.Function):
-    """Bilinear VertexAlign of every map into its column block of an SV x sum(C_m) output; gradients to the maps and to the
-    vertex positions (csrc/vert_align_bilinear.cu)."""
+_MAP_SIZES = {}
+
+
+def _map_size(S: int) -> int:
+    """Address of a host int holding S: the one-entry ``map_size_host`` of a one-map row gather (an int argument keeps the
+    call on the fast path)."""
+    a = _MAP_SIZES.get(S)
+    if a is None:
+        a = _MAP_SIZES[S] = (ctypes.c_int * 1)(S)
+    return ctypes.addressof(a)
+
+
+class _VertAlign(torch.autograd.Function):
+    """VertexAlign of every map into its column block of an SV x sum(C_m) output, on the channels-last fp32 rows of each map
+    (``feature_rows``).  Reference mode: the masked nearest-texel row gather (csrc/align_proj.cu), gradients to the maps
+    only.  Bilinear mode: the bilinear sample of the rows (csrc/vert_align_bilinear.cu), gradients to the maps and to the
+    vertex positions.  Map gradients come back in the map's dtype."""
 
     @staticmethod
-    def forward(ctx, pos, vert_mesh, mesh_info, *fmaps):
+    def forward(ctx, bilinear, pos, vert_mesh, mesh_info, *fmaps):
         pos_c = _f32c(pos.detach())
-        maps = _square_maps(fmaps, "VertexAlign")
+        maps = [_map_tensor(f) for f in fmaps]
         SV = pos_c.shape[0]
         ctot = sum(m.shape[1] for m in maps)
         out = torch.empty(SV, ctot, dtype=torch.float32, device=pos.device)
@@ -1063,11 +1010,16 @@ class _VertAlignBilinear(torch.autograd.Function):
         for m in maps:
             n_img, C, S, _ = m.shape
             r = feature_rows(m)
-            _lib.call("mrb_vert_align_bilinear_fwd", _lib.ptr(r), C, C, S, n_img, _lib.ptr(pos_c), _lib.ptr(vert_mesh),
-                      _lib.ptr(mesh_info), SV, 0, _lib.ptr(out) + 4 * off, ctot)
-            rows.append(r)
+            if bilinear:
+                _lib.call("mrb_vert_align_bilinear_fwd", _lib.ptr(r), C, C, S, n_img, _lib.ptr(pos_c), _lib.ptr(vert_mesh),
+                          _lib.ptr(mesh_info), SV, 0, _lib.ptr(out) + 4 * off, ctot)
+                rows.append(r)
+            else:
+                _lib.call("mrb_vert_align_proj_fwd", _lib.ptr(r), C, 1, _map_size(S), n_img, _lib.ptr(pos_c), _lib.ptr(vert_mesh),
+                          _lib.ptr(mesh_info), SV, _lib.ptr(out) + 4 * off, ctot)
             off += C
         ctx.save_for_backward(pos_c, vert_mesh, mesh_info, *rows)
+        ctx.bilinear = bilinear
         ctx.shapes = [tuple(m.shape) for m in maps]
         ctx.dtypes = [f.dtype for f in fmaps]
         ctx.pos_dtype = pos.dtype
@@ -1077,17 +1029,26 @@ class _VertAlignBilinear(torch.autograd.Function):
     def backward(ctx, gout):
         pos_c, vert_mesh, mesh_info = ctx.saved_tensors[:3]
         rows = ctx.saved_tensors[3:]
-        gout = _rows(gout)
+        gout = _rows(gout)                       # usually a column slice of a stage-input gradient: read in place
         SV, ldg = gout.shape[0], gout.stride(0)
         dev = gout.device
-        gpos = torch.zeros(SV, 3, dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
+        gpos = torch.zeros(SV, 3, dtype=torch.float32, device=dev) if ctx.bilinear and ctx.needs_input_grad[1] else None
         grads, off = [], 0
-        for i, (shape, r) in enumerate(zip(ctx.shapes, rows)):
+        for i, shape in enumerate(ctx.shapes):
             n_img, C, S, _ = shape
-            grows = torch.zeros(r.shape, dtype=torch.float32, device=dev) if ctx.needs_input_grad[3 + i] else None
-            if grows is not None or gpos is not None:
-                _lib.call("mrb_vert_align_bilinear_bwd", gout.data_ptr() + 4 * off, ldg, _lib.ptr(r), C, C, S, n_img,
-                          _lib.ptr(pos_c), _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, _lib.ptr(grows), C, _lib.ptr(gpos), 1)
+            want = ctx.needs_input_grad[4 + i]
+            if ctx.bilinear:
+                grows = torch.zeros(n_img * S * S, C, dtype=torch.float32, device=dev) if want else None
+                if grows is not None or gpos is not None:
+                    _lib.call("mrb_vert_align_bilinear_bwd", gout.data_ptr() + 4 * off, ldg, _lib.ptr(rows[i]), C, C, S, n_img,
+                              _lib.ptr(pos_c), _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, _lib.ptr(grows), C,
+                              _lib.ptr(gpos), 1)
+            elif want:
+                grows = torch.empty(n_img * S * S, C, dtype=torch.float32, device=dev)      # zero-filled by the call
+                _lib.call("mrb_vert_align_proj_bwd", gout.data_ptr() + 4 * off, ldg, C, 1, _map_size(S), n_img,
+                          _lib.ptr(pos_c), _lib.ptr(vert_mesh), _lib.ptr(mesh_info), SV, _lib.ptr(grows))
+            else:
+                grows = None
             if grows is not None:
                 g = torch.empty(shape, dtype=torch.float32, device=dev)
                 _lib.call("mrb_rows_to_feature_map", _lib.ptr(grows), C, n_img, C, S * S, _lib.ptr(g))
@@ -1097,7 +1058,13 @@ class _VertAlignBilinear(torch.autograd.Function):
             off += C
         if gpos is not None and ctx.pos_dtype != torch.float32:
             gpos = gpos.to(ctx.pos_dtype)
-        return (gpos, None, None) + tuple(grads)
+        return (None, gpos, None, None) + tuple(grads)   # reference mode: no gradient to positions (reference layers.py:592)
+
+
+def vert_align(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
+               image_sizes, mesh_index: Sequence[int], topo: Optional[MeshTopology] = None) -> Tensor:
+    vert_mesh, info = align_tables(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index, topo)
+    return _VertAlign.apply(False, vertex_positions, vert_mesh, info, *img_features)
 
 
 def vert_align_bilinear(img_features: Sequence[Tensor], vertex_positions: Tensor, vertices_per_mesh: Sequence[int],
@@ -1106,8 +1073,8 @@ def vert_align_bilinear(img_features: Sequence[Tensor], vertex_positions: Tensor
     ``vertex_positions``.  Same projection and axis convention as ``vert_align``; each square map is then sampled like
     ``grid_sample(align_corners=True, padding_mode="border")`` -- see csrc/vert_align_bilinear.cu for the exact
     definition.  fp32 or bf16 maps; the output and the position gradient are fp32, map gradients come in the map's dtype."""
-    vert_mesh, info = _bilinear_tables(img_features, vertex_positions, vertices_per_mesh, mesh_index, image_sizes)
-    return _VertAlignBilinear.apply(vertex_positions, vert_mesh, info, *img_features)
+    vert_mesh, info = align_tables(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index)
+    return _VertAlign.apply(True, vertex_positions, vert_mesh, info, *img_features)
 
 
 def _project_texels(maps: Sequence[Tensor], w: Tensor, n_img: int):
@@ -1176,7 +1143,7 @@ def _linear_maps(weight: Tensor, fmaps: Sequence[Tensor]):
     """(fp32 weight, maps, n_img) of linear(VertexAlign(maps)) after the shape checks."""
     w = _f32c(weight)
     D, ctot = w.shape
-    maps = _square_maps(fmaps, "VertexAlign+linear")
+    maps = [_map_tensor(f) for f in fmaps]
     n_img = maps[0].shape[0]
     if any(m.shape[0] != n_img for m in maps) or sum(m.shape[1] for m in maps) != ctot:
         raise RuntimeError("VertexAlign+linear: maps %s do not match the %d x %d weight" %
@@ -1195,7 +1162,6 @@ class _VertAlignLinear(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, pos, vert_mesh, mesh_info, weight, *fmaps):
-        _require_cuda(pos, "VertexAlign+linear")
         dev = pos.device
         pos_c = _f32c(pos.detach())
         w, maps, n_img = _linear_maps(weight, fmaps)
@@ -1234,7 +1200,6 @@ class _VertAlignLinearBilinear(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, pos, vert_mesh, mesh_info, weight, *fmaps):
-        _require_cuda(pos, "VertexAlign+linear")
         dev = pos.device
         pos_c = _f32c(pos.detach())
         w, maps, n_img = _linear_maps(weight, fmaps)
@@ -1285,17 +1250,9 @@ def vert_align_linear(img_features: Sequence[Tensor], vertex_positions: Tensor, 
     """``F.linear(VertexAlign()(img_features, ...), weight)`` (weight: out x sum(C_m), no bias) without forming the
     SV x sum(C_m) matrix -- see ``_VertAlignLinear``.  ``bilinear=True``: the same with bilinear VertexAlign
     (``vert_align_bilinear``), differentiable in ``vertex_positions`` too (``_VertAlignLinearBilinear``)."""
+    vert_mesh, info = align_tables(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index, topo)
     if bilinear:
-        vert_mesh, info = _bilinear_tables(img_features, vertex_positions, vertices_per_mesh, mesh_index, image_sizes)
         return _VertAlignLinearBilinear.apply(vertex_positions, vert_mesh, info, weight, *img_features)
-    dev = vertex_positions.device
-    _require_cuda(vertex_positions, "VertexAlign")
-    if sum(int(m) for m in mesh_index) != len(vertices_per_mesh):
-        raise RuntimeError("VertexAlign: sum(mesh_index) must equal the number of meshes")
-    if sum(vertices_per_mesh) != vertex_positions.shape[0]:
-        raise RuntimeError("VertexAlign: vertices_per_mesh does not sum to the number of vertex positions")
-    vert_mesh = vertex_mesh_ids(vertices_per_mesh, vertex_positions.shape[0], dev, topo)
-    info = mesh_info_table(mesh_index, image_sizes, dev)
     return _VertAlignLinear.apply(vertex_positions, vert_mesh, info, weight, *img_features)
 
 

@@ -105,13 +105,18 @@ class VertexAlign(nn.Module):
 
     def forward(self, img_features: List[Tensor], vertex_positions: Tensor, vertices_per_mesh: List[int],
                 image_sizes: List[Tuple[int, int]], mesh_index: List[int]) -> Tensor:
-        if self.training:                                       # layers.py:528-530
-            assert len(vertices_per_mesh) == len(image_sizes)
-            assert list(mesh_index) == [1 for _ in image_sizes]
-        assert len(mesh_index) == len(image_sizes)              # layers.py:532
+        _check_align_call(self, vertices_per_mesh, image_sizes, mesh_index)
         if _bilinear(self):
             return F_.vert_align_bilinear(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index)
         return F_.vert_align(img_features, vertex_positions, vertices_per_mesh, image_sizes, mesh_index)
+
+
+def _check_align_call(align: VertexAlign, vertices_per_mesh, image_sizes, mesh_index) -> None:
+    """The assertions of reference VertexAlign.forward (layers.py:528-532), for the stages that evaluate it fused."""
+    if align.training:
+        assert len(vertices_per_mesh) == len(image_sizes)
+        assert list(mesh_index) == [1 for _ in image_sizes]
+    assert len(mesh_index) == len(image_sizes)
 
 
 def _bilinear(align: VertexAlign) -> bool:
@@ -202,10 +207,7 @@ def _align_and_project(align: "VertexAlign", linear: nn.Linear, img_feature_maps
     """``linear(align(maps, positions, ...))`` of reference meshRCNN/layers.py:151-155 / :226-230."""
     if not FUSE_ALIGN_BOTTLENECK or linear.bias is not None:
         return linear(align(img_feature_maps, vertex_positions, vertice_index, image_sizes, mesh_index))
-    if align.training:                                          # the checks of VertexAlign.forward (layers.py:528-532)
-        assert len(vertice_index) == len(image_sizes)
-        assert list(mesh_index) == [1 for _ in image_sizes]
-    assert len(mesh_index) == len(image_sizes)
+    _check_align_call(align, vertice_index, image_sizes, mesh_index)
     return F_.vert_align_linear(img_feature_maps, vertex_positions, vertice_index, image_sizes, mesh_index, linear.weight,
                                 bilinear=_bilinear(align))
 
@@ -316,10 +318,7 @@ class VertixRefinePix3D(nn.Module):
         mesh_index = _default_mesh_index(mesh_index, image_sizes)
         if FUSE_STAGE_INPUTS and self.graphConv0.w0.shape[1] % 4 == 0 and not _bilinear(self.vertAlign):
             # VertexAlign stays factored: graphConv0 projects the texels and gathers rows (functional.TexelTerm)
-            if self.vertAlign.training:                             # the checks of VertexAlign.forward (layers.py:528-532)
-                assert len(vertice_index) == len(image_sizes)
-                assert list(mesh_index) == [1 for _ in image_sizes]
-            assert len(mesh_index) == len(image_sizes)
+            _check_align_call(self.vertAlign, vertice_index, image_sizes, mesh_index)
             # (the registered topology of a Cubify adjacency already holds the per-vertex mesh ids)
             aligned = F_.TexelTerm(back_bone_features, vertex_positions, vertice_index, image_sizes, mesh_index,
                                    topo=topology.lookup(vertex_adjacency, vertex_positions.shape[0]))

@@ -17,13 +17,14 @@ from . import _lib
 
 class MeshTopology:
     """CSR adjacency (row-sorted, int32) of a packed batch of meshes, plus the CSR of its transpose (the
-    backward of the neighbour sum gathers along columns; for symmetric adjacency both are the same arrays)."""
+    backward of the neighbour sum gathers along columns; for symmetric adjacency both are the same arrays).
+    Cubify also records the per-vertex mesh ids ``vert_mesh`` and the per-mesh vertex counts ``v_index`` they belong to."""
 
     __slots__ = ("num_vertices", "num_edges", "rowptr", "col", "rowptr_t", "col_t", "symmetric", "vert_mesh",
-                 "v_offsets", "row32", "bad_index_flags", "__weakref__")
+                 "v_index", "v_offsets", "row32", "bad_index_flags", "__weakref__")
 
     def __init__(self, num_vertices, num_edges, rowptr, col, rowptr_t=None, col_t=None, symmetric=False,
-                 vert_mesh=None, v_offsets=None, row32=None):
+                 vert_mesh=None, v_offsets=None, row32=None, v_index=None):
         self.num_vertices = int(num_vertices)
         self.num_edges = int(num_edges)
         self.rowptr = rowptr
@@ -32,6 +33,7 @@ class MeshTopology:
         self.rowptr_t = rowptr if symmetric else rowptr_t
         self.col_t = col if symmetric else col_t
         self.vert_mesh = vert_mesh
+        self.v_index = None if v_index is None else list(v_index)
         self.v_offsets = v_offsets
         self.row32 = row32
         self.bad_index_flags = None      # device flags of mrb_coo_to_csr (foreign COO tensors only)
